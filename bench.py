@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- HW1F path-steps/s on the BASELINE.json headline workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch: the Q1 bond-curve workload of
@@ -361,13 +361,14 @@ def run_reference_arm(args, rank, real_stdout):
                        "l2": "not flushed (the reference re-reads its own 50 MB state array every step)",
                        "parallelism": "single GPU on rank 0 (the reference has no multi-GPU path)"}}
     if os.path.exists(harness):
-        out = os.path.join(ROOT, "gpurun_out", "ref_bench_q1.json")
-        os.makedirs(os.path.dirname(out), exist_ok=True)
+        import tempfile
         env = dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0])
-        subprocess.run([harness, "bench", "q1", str(args.steps), str(args.warmup), out], check=True, env=env,
-                       stdout=subprocess.DEVNULL, timeout=1800)
-        with open(out) as f:
-            r = json.load(f)
+        with tempfile.TemporaryDirectory() as td:     # the tree may be read-only
+            out = os.path.join(td, "ref_bench_q1.json")
+            subprocess.run([harness, "bench", "q1", str(args.steps), str(args.warmup), out], check=True, env=env,
+                           stdout=subprocess.DEVNULL, timeout=1800)
+            with open(out) as f:
+                r = json.load(f)
         ms = r["workload_ms_per_step"]
         value = r["path_steps_per_step"] / (ms * 1e-3)
         line.update({"value": value, "ms_per_step": ms, "gpu_launches": 3 * args.steps,
@@ -423,7 +424,14 @@ def main():
                     help="moment all-reduce for N > 1: own NVLink peer-memory kernel (hw1f_comm_*) or NCCL")
     ap.add_argument("--mode", default="decomposed", choices=["decomposed", "reference_order"],
                     help="simulation arithmetic (include/hw1f.h HW1F_MODE_*); both give the same Gaussians")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last device-timed step computed to DIR/*.npy: the moment vector "
+                         "(moments.npy, float64) and the P, f, P_se it finishes to (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs writes the engine's outputs (--impl engine)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -538,6 +546,13 @@ def main():
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
     ms_per_step = float(total_ms.item()) / args.steps
     value = path_steps_per_step / (ms_per_step * 1e-3)
+
+    # what the last timed step computed (seed 5000 + steps - 1, so the same arguments give the same inputs), taken
+    # before later steps overwrite the moment vector
+    dumped = None
+    if args.dump_outputs:
+        dumped = {"moments": moments.cpu().numpy()}
+        dumped.update(eng.bond_curve_finish(moments.data_ptr(), n_paths * world))
 
     # ---- end-to-end region: public host-buffer API, wall clock between synchronisations ----
     def timed_e2e(loop):
@@ -798,6 +813,10 @@ def main():
                   "multi_gpu": multi_check},
         "published_v100_path_steps_per_s": 3.91e11,
     }
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     _emit(line, real_stdout)
     if world > 1:
         dist.destroy_process_group()
