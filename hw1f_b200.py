@@ -15,6 +15,7 @@ Engine = _pkg.Engine
 Rng = _pkg.Rng
 HW1FError = _pkg.HW1FError
 default_params = _pkg.default_params
+caplet_schedule = _pkg.caplet_schedule
 Params = _pkg.Params
 LIB_PATH = _pkg.LIB_PATH
 _ffi = _pkg._ffi

@@ -255,6 +255,56 @@ int hw1f_vega_pathwise_batch(hw1f_engine* eng, const uint64_t* seeds, int32_t n_
                              float S1, float S2, float K, const float* P_mkt, const float* f_mkt,
                              int32_t n_steps_S1, float* vega, float* sim_ms);
 
+/* ---- caps and floors: a strip of caplets in one simulation pass -------------------------- */
+/* No reference call site: the reference prices one bond call (hw1f_zbc_cv).  A cap is a strip of zero-coupon bond PUTS,
+ * a floor a strip of bond CALLS, one per reset date; one launch prices every caplet of the strip on one set of paths
+ * (each path is stepped once to the last reset step and evaluated at every reset step on the way) and returns the
+ * moments of each caplet and of the whole strip, in both arithmetic modes and at any normal offset.
+ * The ABI speaks in bonds: a caplet on the rate L(T_r, T_p) with strike rate kappa, accrual tau and notional M equals
+ * N ZBP(T_r, T_p, K) with K = 1 / (1 + tau kappa) and N = M (1 + tau kappa); a floorlet is the same with ZBC (the
+ * Python layer's caplet_schedule() converts rates). */
+typedef struct hw1f_caplet {
+    float T_reset;          /* option expiry = reset date T_r (> 0)                                   */
+    float T_pay;            /* bond maturity = payment date T_p, T_reset < T_pay <= T_final           */
+    float K;                /* bond strike (> 0)                                                      */
+    float N;                /* multiplier (> 0): payoff N (K - P)^+ for a cap, N (P - K)^+ for a floor */
+    int32_t n_steps_reset;  /* step at which r is read; < 0: the step nearest to T_reset / dt          */
+    int32_t reserved;
+} hw1f_caplet;
+
+/* Moments over antithetic PAIRS: X = x(+G) + x(-G), Y = y(+G) + y(-G) for each of the n_pairs = n_paths subsequences,
+ * and every statistic is over the n_pairs samples of the pair means X/2, Y/2 (price_raw = sum X / (2 n_pairs),
+ * se_raw = sqrt(var(X/2) / n_pairs)).  This differs from hw1f_zbc_result, whose second moments follow the reference
+ * (per-twin sums, the twins treated as independent samples): these standard errors are honest. */
+typedef struct hw1f_cap_result {   /* one caplet, or the whole strip */
+    double mom[5];          /* sum X, sum Y, sum X^2, sum Y^2, sum XY over antithetic PAIRS: X = x(+G) + x(-G) */
+    double price_raw, se_raw;
+    double price_cv, se_cv; /* optimal-beta control variate, control Y = N D(T_r) P(T_r, T_p)             */
+    double beta, corr;
+    double control_mean;    /* known mean of the control: N P_mkt(T_p) interpolated like interp_mkt; summed for the strip */
+} hw1f_cap_result;
+
+#define HW1F_KIND_CAP 0
+#define HW1F_KIND_FLOOR 1
+#define HW1F_MAX_CAPLETS 100   /* 5 (100 + 1) = 505 doubles: fits the peer mailboxes (kCommMaxCount = 512) */
+
+/* Reset steps ROUND to the nearest step (n_steps_reset < 0: lround(T_reset / dt) in double), unlike hw1f_steps_to, which
+ * reproduces the reference's truncation for parity: a product date a hair below a step would otherwise move a reset by a
+ * whole step.  HW1F_ERR_INVALID if |T_reset - k dt| > 1e-3 dt.
+ * Every argument is checked before any launch; HW1F_ERR_INVALID (with a message) for: a kind other than HW1F_KIND_*,
+ * n_caplets outside [1, HW1F_MAX_CAPLETS], reset steps that decrease along the strip or lie outside [1, n_steps],
+ * T_pay <= T_reset or T_pay > T_final, K or N not finite and positive.  After a failure the rng has not moved and no
+ * kernel was launched.
+ * The strip's price uses ONE beta on Y_strip = sum_i Y_i; its price_raw is the sum of the caplets' up to rounding. */
+/* out[n_caplets + 1]: the caplets in order, then the strip.  Advances rng by the last reset step. */
+int hw1f_cap_floor(hw1f_engine* eng, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caplets, int32_t n_caplets,
+                   const float* P_mkt, const float* f_mkt, hw1f_cap_result* out, float* sim_ms);
+/* split form, like every other estimator: d_moments[5 (n_caplets + 1)] on the device; honours hw1f_comm_attach */
+int hw1f_cap_floor_moments(hw1f_engine* eng, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caplets, int32_t n_caplets,
+                           const float* P_mkt, const float* f_mkt, double* d_moments);
+int hw1f_cap_floor_finish(hw1f_engine* eng, const double* d_moments, uint64_t n_paths_total, const hw1f_caplet* caplets,
+                          int32_t n_caplets, const float* P_mkt, hw1f_cap_result* out);
+
 /* ---- fused pass (BASELINE.json scaling run) --------------------------------------------- */
 /* One launch: antithetic curve sums on the maturity grid + ZBC/control moments + pathwise-vega
  * tangent (both antithetic twins) evaluated at step n_steps_S1, all on the same normals.

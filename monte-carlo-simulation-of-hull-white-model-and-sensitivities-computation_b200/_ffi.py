@@ -11,6 +11,8 @@ OK = 0
 MODE_REFERENCE_ORDER, MODE_DECOMPOSED = 0, 1
 ASYNC_SLOTS = 4   # HW1F_ASYNC_SLOTS
 ERR_INVALID, ERR_CUDA, ERR_NO_DEVICE, ERR_UNSUPPORTED, ERR_NO_MODEL, ERR_COMM = 1, 2, 3, 4, 5, 6
+KIND_CAP, KIND_FLOOR = 0, 1   # HW1F_KIND_*
+MAX_CAPLETS = 100             # HW1F_MAX_CAPLETS
 
 
 class Params(C.Structure):
@@ -55,6 +57,24 @@ class VegaResult(C.Structure):
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_}
+
+
+class Caplet(C.Structure):
+    """hw1f_caplet: one zero-coupon bond option of a cap (put) or floor (call) strip."""
+    _fields_ = [("T_reset", C.c_float), ("T_pay", C.c_float), ("K", C.c_float), ("N", C.c_float),
+                ("n_steps_reset", C.c_int32), ("reserved", C.c_int32)]
+
+
+class CapResult(C.Structure):
+    """hw1f_cap_result: one caplet, or the whole strip (moments over antithetic pairs)."""
+    _fields_ = [("mom", C.c_double * 5), ("price_raw", C.c_double), ("se_raw", C.c_double),
+                ("price_cv", C.c_double), ("se_cv", C.c_double), ("beta", C.c_double), ("corr", C.c_double),
+                ("control_mean", C.c_double)]
+
+    def as_dict(self):
+        d = {n: getattr(self, n) for n, _ in self._fields_ if n != "mom"}
+        d["mom"] = list(self.mom)
+        return d
 
 
 # every symbol include/hw1f.h declares: name -> (restype, argtypes)
@@ -107,6 +127,9 @@ SYMBOLS = {
                             C.POINTER(VegaResult)]),
     "hw1f_vega_pathwise_batch": (C.c_int, [_P, _P, C.c_int32, C.c_uint64, C.c_float, C.c_float, C.c_float, _P, _P,
                                            C.c_int32, _P, _F]),
+    "hw1f_cap_floor": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.POINTER(CapResult), _F]),
+    "hw1f_cap_floor_moments": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
+    "hw1f_cap_floor_finish": (C.c_int, [_P, _P, C.c_uint64, _P, C.c_int32, _P, C.POINTER(CapResult)]),
     "hw1f_fused_moments": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_int32, _P]),
     "hw1f_fused_fd_moments": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_float, C.c_int32, _P]),
     "hw1f_fused": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_float, C.c_int32, _P, _P, _P,

@@ -6,6 +6,7 @@
 // fails the entry point returns an error code and hw1f_last_error() says why.
 #include "../../include/hw1f.h"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -18,6 +19,7 @@
 #include "hw1f_kernels.cuh"
 #include "hw1f_kernels_extra.cuh"
 #include "hw1f_kernels_fast.cuh"
+#include "hw1f_kernels_cap.cuh"
 #include "hw1f_tail.cuh"
 #include "hw1f_probe.cuh"
 #include "xorwow_jump.hpp"
@@ -105,6 +107,7 @@ struct hw1f_engine {
     DevBuf<float2> d_state;              // dumped noise state (h, q) per subsequence (recalibrated FD, one pass)
     DevBuf<double> d_moments;            // internal moment vector
     DevBuf<float> d_out;                 // epilogue outputs
+    DevBuf<char> d_cap;                  // hw1f_cap_floor*: caplet table + market curves, one staged upload per call
     DevBuf<int> d_int;
     void* h_stage = nullptr;             // pinned
     size_t h_stage_bytes = 0;
@@ -969,6 +972,8 @@ int init_kernels(hw1f_engine* e)
     HW_CUDA(e, opt_in(zbc_sum_kernel<1>, b));
     HW_CUDA(e, opt_in(zbc_sum_kernel<2>, b));
     HW_CUDA(e, opt_in(zbc_sum_kernel<3>, b));
+    HW_CUDA(e, opt_in(cap_kernel<0>, b));
+    HW_CUDA(e, opt_in(cap_kernel<1>, b));
     // the small kernels have no dynamic shared memory; querying them loads their code now instead
     // of inside the first timed call
     cudaFuncAttributes attr;
@@ -1102,7 +1107,7 @@ int hw1f_engine_destroy(hw1f_engine* e)
     for (auto& d : e->d_drift) d.release();
     e->d_mkt.release(); e->d_center.release(); e->d_plans.release();
     for (auto& d : e->d_emI) d.release(); e->d_partials.release(); e->d_moments.release(); e->d_state.release();
-    e->d_out.release(); e->d_int.release();
+    e->d_out.release(); e->d_int.release(); e->d_cap.release();
     e->d_model.release();
     e->d_fd.release();
     e->d_tail_cnt.release(); e->d_gpart.release();
@@ -2198,6 +2203,180 @@ int hw1f_fused(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const
     HW_CUDA(e, cudaEventElapsedTime(&ms, e->ev0, e->ev1));
     vega->ms_pathwise = vega->ms_fd = ms;
     if (sim_ms) *sim_ms = ms;
+    return HW1F_OK;
+}
+
+// ---- caps and floors ------------------------------------------------------------------------------
+// every argument checked before any launch; steps[i] = the resolved reset step of caplet i
+static int cap_validate(hw1f_engine* e, int32_t kind, const hw1f_caplet* caps, int32_t n, std::vector<int>& steps)
+{
+    HW_REQUIRE(e, kind == HW1F_KIND_CAP || kind == HW1F_KIND_FLOOR, "kind must be HW1F_KIND_CAP or HW1F_KIND_FLOOR");
+    HW_REQUIRE(e, n >= 1 && n <= HW1F_MAX_CAPLETS, "n_caplets must be in [1, HW1F_MAX_CAPLETS]");
+    steps.assign(n, 0);
+    const double dt = (double)e->dt;
+    for (int i = 0; i < n; ++i) {
+        const hw1f_caplet& c = caps[i];
+        const std::string at = " (caplet " + std::to_string(i) + ")";
+        HW_REQUIRE(e, std::isfinite(c.T_reset) && c.T_reset > 0.0f, "T_reset must be finite and positive" + at);
+        HW_REQUIRE(e, std::isfinite(c.T_pay) && c.T_pay > c.T_reset, "T_pay must be greater than T_reset" + at);
+        HW_REQUIRE(e, c.T_pay <= e->p.T_final, "T_pay must not exceed T_final" + at);
+        HW_REQUIRE(e, std::isfinite(c.K) && c.K > 0.0f, "K must be finite and positive" + at);
+        HW_REQUIRE(e, std::isfinite(c.N) && c.N > 0.0f, "N must be finite and positive" + at);
+        long k = c.n_steps_reset;
+        if (k < 0) {
+            // nearest step, not truncation: a date a hair below a step must not move the reset by a whole step
+            k = std::lround((double)c.T_reset / dt);
+            HW_REQUIRE(e, std::fabs((double)c.T_reset - (double)k * dt) <= 1e-3 * dt,
+                       "T_reset is not on the step grid (|T_reset - k dt| > 1e-3 dt): pass n_steps_reset" + at);
+        }
+        HW_REQUIRE(e, k >= 1 && k <= e->p.n_steps, "reset step outside [1, n_steps]" + at);
+        HW_REQUIRE(e, i == 0 || k >= steps[i - 1], "reset steps must be non-decreasing along the strip" + at);
+        steps[i] = (int)k;
+    }
+    return HW1F_OK;
+}
+
+// one staged upload of [caplet table | P_mkt | f_mkt], the launch and its tail
+static int cap_run(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n,
+                   const std::vector<int>& steps, const float* P_mkt, const float* f_mkt, double* d_moments,
+                   const Finish& fin)
+{
+    const int nm = e->p.n_mat, nq = 5 * (n + 1);
+    const size_t tab = ((size_t)n * sizeof(CapletDev) + 255) & ~(size_t)255;
+    std::vector<char> h(tab + 2 * (size_t)nm * sizeof(float), 0);
+    CapletDev* cd = reinterpret_cast<CapletDev*>(h.data());
+    for (int i = 0; i < n; ++i) {
+        cd[i].T_reset = caps[i].T_reset;
+        cd[i].T_pay = caps[i].T_pay;
+        cd[i].K = caps[i].K;
+        cd[i].N = caps[i].N;
+        cd[i].m = (float)e->det_m[0][steps[i]];
+        cd[i].Im = (float)e->det_I[0][steps[i]];
+        cd[i].step = steps[i];
+        cd[i].pad = 0;
+    }
+    memcpy(h.data() + tab, P_mkt, nm * sizeof(float));
+    memcpy(h.data() + tab + nm * sizeof(float), f_mkt, nm * sizeof(float));
+    const int decomp = e->mode == HW1F_MODE_DECOMPOSED;
+    const size_t smem = cap_smem_bytes(decomp, n, steps[n - 1]);
+    HW_TRY(decomp ? set_smem(e, cap_kernel<1>, smem) : set_smem(e, cap_kernel<0>, smem));
+    HW_CUDA(e, e->d_cap.ensure(h.size()));
+    HW_TRY(upload(e, e->d_cap.p, h.data(), h.size()));
+    Launch L;
+    HW_TRY(prepare_launch(e, &rng->seed, 1, rng->first_path, rng->n_paths, rng->offset, &L));
+    HW_CUDA(e, e->d_partials.ensure((size_t)L.grid_x * nq));
+    const ScenDev sc = scen_dev(e, e->p.sigma, e->sig_st, 0);
+    const CapletDev* d_caps = reinterpret_cast<const CapletDev*>(e->d_cap.p);
+    const float* d_P = reinterpret_cast<const float*>(e->d_cap.p + tab);
+    const float sgn = (kind == HW1F_KIND_CAP) ? -1.0f : 1.0f;
+    HW_CUDA(e, launch_k(decomp ? cap_kernel<1> : cap_kernel<0>, dim3(L.grid_x, 1), kThreads, smem, e->stream, true, L.g,
+                        L.seeds, model_dev(e), sc, d_caps, (int)n, d_P, d_P + nm, sgn, L.lead, e->d_partials.p));
+    HW_TRY(check_launch(e, "cap_kernel"));
+    HW_TRY(launch_tail(e, L, L.g.n_paths, nq, 0, nullptr, nullptr, 0.f, d_moments, nq, nq, fin));
+    rng->offset += (uint64_t)steps[n - 1];
+    return HW1F_OK;
+}
+
+// P_mkt(T) as interp_mkt evaluates it on the device (IEEE single operations, one fused multiply-add each)
+static float host_interp_mkt(const hw1f_engine* e, const float* data, float T)
+{
+    const int n = e->p.n_mat;
+    const float inv = 1.0f / e->spacing;
+    const float prod = T * inv;
+    const int idx = (prod >= (float)n) ? n : (int)prod;
+    if (idx >= n - 1) return data[n - 1];
+    const float al = std::fmaf((float)idx, -e->spacing, T) * inv;
+    const float om = 1.0f - al;
+    return std::fmaf(data[idx], om, al * data[idx + 1]);
+}
+
+// double algebra on the pair moments: n_pairs samples of the pair means x = X/2, y = Y/2
+static void cap_algebra(const double mom[5], uint64_t n_pairs, double control_mean, hw1f_cap_result* r)
+{
+    memset(r, 0, sizeof(*r));
+    for (int k = 0; k < 5; ++k) r->mom[k] = mom[k];
+    const double n = (double)n_pairs;
+    const double sx = 0.5 * mom[0], sy = 0.5 * mom[1], sxx = 0.25 * mom[2], syy = 0.25 * mom[3], sxy = 0.25 * mom[4];
+    const double mx = sx / n, my = sy / n;
+    const double d = n > 1.0 ? n - 1.0 : 1.0;
+    double vxx = (sxx - sx * mx) / d, vyy = (syy - sy * my) / d;
+    const double cxy = (sxy - sx * my) / d;
+    if (vxx < 0.0) vxx = 0.0;
+    if (vyy < 0.0) vyy = 0.0;
+    const double beta = vyy > 0.0 ? cxy / vyy : 0.0;
+    double vcv = vxx - 2.0 * beta * cxy + beta * beta * vyy;
+    if (vcv < 0.0) vcv = 0.0;
+    r->price_raw = mx;
+    r->se_raw = sqrt(vxx / n);
+    r->beta = beta;
+    r->price_cv = mx - beta * (my - control_mean);
+    r->se_cv = sqrt(vcv / n);
+    r->corr = (vxx > 0.0 && vyy > 0.0) ? cxy / sqrt(vxx * vyy) : 0.0;
+    r->control_mean = control_mean;
+}
+
+static void cap_results(const hw1f_engine* e, const double* mom, uint64_t n_pairs, const hw1f_caplet* caps, int32_t n,
+                        const float* P_mkt, hw1f_cap_result* out)
+{
+    double strip_mean = 0.0;
+    for (int i = 0; i < n; ++i) {
+        const double cm = (double)caps[i].N * (double)host_interp_mkt(e, P_mkt, caps[i].T_pay);
+        strip_mean += cm;
+        cap_algebra(mom + 5 * i, n_pairs, cm, out + i);
+    }
+    cap_algebra(mom + 5 * n, n_pairs, strip_mean, out + n);
+}
+
+int hw1f_cap_floor_moments(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n,
+                           const float* P_mkt, const float* f_mkt, double* d_moments)
+{
+    HW_TRY(require_model(e));
+    if (!rng || !caps || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    HW_TRY(cap_validate(e, kind, caps, n, steps));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    Finish fin;
+    fin.exchange = true;   // with peers attached (hw1f_comm_attach) the last block all-reduces the vector itself
+    return cap_run(e, rng, kind, caps, n, steps, P_mkt, f_mkt, d_moments, fin);
+}
+
+int hw1f_cap_floor_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths_total, const hw1f_caplet* caps,
+                          int32_t n, const float* P_mkt, hw1f_cap_result* out)
+{
+    HW_TRY(require_model(e));
+    if (!d_moments || !caps || !P_mkt || !out) return HW1F_ERR_INVALID;
+    HW_REQUIRE(e, n_paths_total >= 1 && n_paths_total < (1ull << 40), "n_paths_total outside [1, 2^40)");
+    std::vector<int> steps;
+    HW_TRY(cap_validate(e, HW1F_KIND_CAP, caps, n, steps));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    std::vector<double> mom(5 * (size_t)(n + 1));
+    HW_TRY(download(e, mom.data(), d_moments, mom.size() * sizeof(double)));
+    HW_TRY(require_finite(e, mom.data(), (int)mom.size()));
+    cap_results(e, mom.data(), n_paths_total, caps, n, P_mkt, out);
+    return HW1F_OK;
+}
+
+int hw1f_cap_floor(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n, const float* P_mkt,
+                   const float* f_mkt, hw1f_cap_result* out, float* sim_ms)
+{
+    HW_TRY(require_model(e));
+    if (!rng || !caps || !P_mkt || !f_mkt || !out) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    HW_TRY(cap_validate(e, kind, caps, n, steps));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    const size_t nq = 5 * (size_t)(n + 1);
+    HW_CUDA(e, e->d_moments.ensure(std::max(4 * (size_t)e->p.n_mat * kMaxRuns, nq)));
+    HW_TRY(warm_geometry(e, rng));
+    Finish fin;
+    fin.host_mom = res_mom(e, 0);   // the result area holds at least 512 doubles
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev0, e->stream));
+    HW_TRY(cap_run(e, rng, kind, caps, n, steps, P_mkt, f_mkt, e->d_moments.p, fin));
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev1, e->stream));
+    HW_TRY(wait_results(e));
+    std::vector<double> mom(res_mom(e, 0), res_mom(e, 0) + nq);
+    HW_TRY(require_finite(e, mom.data(), (int)nq));
+    cap_results(e, mom.data(), rng->n_paths, caps, n, P_mkt, out);
+    if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
     return HW1F_OK;
 }
 

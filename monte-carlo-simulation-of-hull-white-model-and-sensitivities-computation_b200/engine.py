@@ -8,7 +8,7 @@ import ctypes as C
 import numpy as np
 
 from . import _ffi
-from ._ffi import Constants, Params, VegaResult, ZbcResult
+from ._ffi import CapResult, Caplet, Constants, Params, VegaResult, ZbcResult
 
 
 class HW1FError(RuntimeError):
@@ -37,6 +37,68 @@ def _f32(a, n=None):
 
 def _ptr(a):
     return a.ctypes.data_as(C.c_void_p)
+
+
+# numpy mirror of hw1f_caplet
+CAPLET_DTYPE = np.dtype([(n, np.float32 if t is C.c_float else np.int32) for n, t in Caplet._fields_])
+assert CAPLET_DTYPE.itemsize == C.sizeof(Caplet)
+
+
+def caplet_schedule(resets, pays, strike_rate, notional=1.0):
+    """Caplets on the simple rates L(T_r, T_p) struck at `strike_rate` (scalar or one per caplet), as the bond options
+    the engine prices: a caplet pays M tau (L - kappa)^+ at T_p, which is worth N ZBP(T_r, T_p, K) with tau = T_p - T_r,
+    K = 1 / (1 + tau kappa) and N = M (1 + tau kappa) (a floorlet: N ZBC).  Reset steps are left to the engine
+    (n_steps_reset = -1: the step nearest to T_r / dt).  Returns a structured array of hw1f_caplet; no GPU needed."""
+    resets = np.atleast_1d(np.asarray(resets, np.float64))
+    pays = np.atleast_1d(np.asarray(pays, np.float64))
+    if resets.shape != pays.shape:
+        raise ValueError("resets and pays must have the same length")
+    kappa = np.broadcast_to(np.asarray(strike_rate, np.float64), resets.shape)
+    M = np.broadcast_to(np.asarray(notional, np.float64), resets.shape)
+    tau = pays - resets
+    grow = 1.0 + tau * kappa
+    out = np.zeros(resets.shape, CAPLET_DTYPE)
+    out["T_reset"], out["T_pay"] = resets, pays
+    out["K"], out["N"] = 1.0 / grow, M * grow
+    out["n_steps_reset"] = -1
+    return out
+
+
+def _caplets(caplets):
+    """structured array of hw1f_caplet (caplet_schedule), a ctypes Caplet array, or a sequence of Caplet / dicts"""
+    if isinstance(caplets, np.ndarray) and caplets.dtype.names:
+        a = np.zeros(caplets.shape, CAPLET_DTYPE)
+        for n in CAPLET_DTYPE.names:
+            if n in caplets.dtype.names:
+                a[n] = caplets[n]
+            elif n == "n_steps_reset":
+                a[n] = -1
+        return np.ascontiguousarray(a.ravel())
+    rows = []
+    for c in caplets:
+        if isinstance(c, Caplet):
+            rows.append(tuple(getattr(c, n) for n in CAPLET_DTYPE.names))
+        else:
+            rows.append((c["T_reset"], c["T_pay"], c["K"], c["N"], c.get("n_steps_reset", -1), 0))
+    return np.array(rows, CAPLET_DTYPE)
+
+
+def _kind(kind):
+    if kind in ("cap", _ffi.KIND_CAP):
+        return _ffi.KIND_CAP
+    if kind in ("floor", _ffi.KIND_FLOOR):
+        return _ffi.KIND_FLOOR
+    return int(kind) if isinstance(kind, (int, np.integer)) else -1   # the engine rejects it with a message
+
+
+def _cap_results(res, n):
+    """per-caplet numpy arrays and the strip as a dict"""
+    rows = [res[i].as_dict() for i in range(n)]
+    out = {k: np.array([r[k] for r in rows], np.float64)
+           for k in ("price_cv", "se_cv", "price_raw", "se_raw", "beta", "corr", "control_mean")}
+    out["mom"] = np.array([r["mom"] for r in rows], np.float64).reshape(n, 5)
+    out["strip"] = res[n].as_dict()
+    return out
 
 
 class Rng:
@@ -259,6 +321,34 @@ class Engine:
                                                 self.K_DEFAULT if K is None else K, _ptr(P_mkt), _ptr(f_mkt),
                                                 n_steps_S1, res, C.byref(ms)))
         return [r.as_dict() for r in res], ms.value
+
+    # -- caps and floors: every caplet of a strip in one simulation pass (no reference call site) --
+    def cap_floor(self, rng, caplets, P_mkt, f_mkt, kind="cap"):
+        """kind "cap" (bond puts) or "floor" (bond calls); caplets as from caplet_schedule().  Per-caplet arrays
+        price_cv, se_cv, price_raw, se_raw, beta, corr, control_mean, mom[n, 5], the whole strip under "strip"."""
+        cap = _caplets(caplets)
+        P_mkt, f_mkt = _f32(P_mkt, self.n_mat), _f32(f_mkt, self.n_mat)
+        res, ms = (CapResult * (len(cap) + 1))(), C.c_float()
+        self._check(self._lib.hw1f_cap_floor(self._h, rng._h, _kind(kind), _ptr(cap), len(cap), _ptr(P_mkt), _ptr(f_mkt),
+                                             res, C.byref(ms)))
+        out = _cap_results(res, len(cap))
+        out["sim_ms"] = ms.value
+        return out
+
+    def cap_floor_moments(self, rng, caplets, P_mkt, f_mkt, d_moments_ptr, kind="cap"):
+        """async: device pointer to 5 * (len(caplets) + 1) doubles"""
+        cap = _caplets(caplets)
+        P_mkt, f_mkt = _f32(P_mkt, self.n_mat), _f32(f_mkt, self.n_mat)
+        self._check(self._lib.hw1f_cap_floor_moments(self._h, rng._h, _kind(kind), _ptr(cap), len(cap), _ptr(P_mkt),
+                                                     _ptr(f_mkt), C.c_void_p(d_moments_ptr)))
+
+    def cap_floor_finish(self, d_moments_ptr, n_paths_total, caplets, P_mkt):
+        cap = _caplets(caplets)
+        P_mkt = _f32(P_mkt, self.n_mat)
+        res = (CapResult * (len(cap) + 1))()
+        self._check(self._lib.hw1f_cap_floor_finish(self._h, C.c_void_p(d_moments_ptr), int(n_paths_total), _ptr(cap),
+                                                    len(cap), _ptr(P_mkt), res))
+        return _cap_results(res, len(cap))
 
     # -- Q3 (src/3_sensitivity_analysis.cu) --
     def vega_pathwise(self, rng, P_mkt, f_mkt, S1=5.0, S2=10.0, K=None, n_steps_S1=-1):
