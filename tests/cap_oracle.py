@@ -57,6 +57,17 @@ def _p(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
+def moment_bound(ref, rel=3e-6, eps=2.4e-7):
+    """Largest |engine - oracle| allowed per moment of cap_moments() (same [n + 1, 5] layout): `rel` relative, plus
+    what MUFU.EX2 (the engine) vs exp2f (the oracle) may leave in the payoff.  P = A ex2(..) differs by up to eps
+    relative, so x = D (K - P)^+ inherits an ABSOLUTE error |dx| <= eps y.  Summed over pairs that gives eps sY for
+    sum X, and 2 x dx + dx^2 <= 2 eps x y + eps^2 y^2 for sum X^2 (the square term matters only when every pair of a
+    tiny run is at the money and the oracle's x is zero), eps sYY for sum XY.  The controls get no slack."""
+    sX, sY, sXX, sYY, sXY = np.asarray(ref).T
+    slack = np.stack([eps * sY, 0 * sY, 2 * eps * sXY + eps * eps * sYY, 0 * sY, eps * sYY], axis=1)
+    return rel * np.abs(ref) + slack
+
+
 def cap_moments(oracle: Oracle, seed, n_pairs, caplets, P_mkt, f_mkt, kind="cap", first_path=0, offset=0, sigma=None):
     """moments[n + 1, 5] over antithetic pairs on the model of `oracle`; caplets: any structured array with T_reset,
     T_pay, K, N and optionally n_steps_reset (< 0 or absent: the step nearest to T_reset / dt)"""

@@ -278,13 +278,16 @@ def test_finish_beyond_int_range(engine, hw, curve):
 
 
 @pytest.mark.parametrize("call", ["zbc_cv", "vega_pathwise", "vega_fd", "vega_fd_recalibrated", "vega", "fused",
-                                  "zbc_cv_batch", "vega_pathwise_batch", "sample_paths", "theta"])
+                                  "zbc_cv_batch", "vega_pathwise_batch", "sample_paths", "theta", "cap_floor",
+                                  "cap_floor_moments"])
 def test_every_entry_point_as_first_call_of_a_fresh_engine(engine, hw, curve, call):
     """lazily built state (jump tables, window tables, bumped-sigma arena, scratch) must not depend on what ran
     before: each entry point, called FIRST on a new engine with a ragged path count, reproduces the long-lived
     session engine bit for bit"""
     n = (1 << 12) + 77
     P, f = curve["P"], curve["f"]
+    resets = 0.25 * np.arange(1, 40)
+    caps = hw.caplet_schedule(resets, resets + 0.25, 0.02)
 
     def run(e):
         if call == "zbc_cv":
@@ -311,6 +314,16 @@ def test_every_entry_point_as_first_call_of_a_fresh_engine(engine, hw, curve, ca
             return list(v)
         if call == "sample_paths":
             return list(e.sample_paths(hw.Rng(SEED, n), 4).ravel())
+        if call == "cap_floor":
+            r = e.cap_floor(hw.Rng(SEED, n).seek(1), caps, P, f, kind="cap")
+            return list(r["mom"].ravel()) + r["strip"]["mom"] + list(r["price_cv"])
+        if call == "cap_floor_moments":
+            import torch
+            m = torch.zeros(5 * (len(caps) + 1), dtype=torch.float64, device="cuda")
+            torch.cuda.synchronize()
+            e.cap_floor_moments(hw.Rng(SEED, n).seek(1), caps, P, f, m.data_ptr(), kind="floor")
+            e.synchronize()
+            return m.cpu().tolist()
         return list(e.theta_calibrate(f)["theta_rec"])
 
     fresh = hw.Engine(device=0)

@@ -380,7 +380,12 @@ def test_grid_stride_chunks_large_run(engine, hw, curve):
     """more chunks than resident blocks: blocks stride over chunks and fold them into their double
     accumulators; the result must equal the sum of shards that each fit in one pass"""
     import torch
-    n = (1 << 22) + 3                         # 8193 chunks of 512 > the 32*SMs grid cap
+    grid = 32 * torch.cuda.get_device_properties(0).multi_processor_count      # prepare_launch's grid cap
+    n = (2 * grid + 37) * 1024 + 3            # chunks of kChunk = 1024 subsequences
+    n_chunks = (n + 1023) // 1024
+    assert n_chunks > 2 * grid                # every block folds 2 or 3 chunks
+    counts = [grid * 1024, grid * 1024, n - 2 * grid * 1024]     # shards of <= grid chunks: one pass each
+    assert all((c + 1023) // 1024 <= grid for c in counts)
     full = torch.zeros(202, dtype=torch.float64, device="cuda")
     torch.cuda.synchronize()
     engine.bond_curve_moments(hw.Rng(99, n), full.data_ptr())
@@ -388,11 +393,11 @@ def test_grid_stride_chunks_large_run(engine, hw, curve):
     part = torch.zeros(202, dtype=torch.float64, device="cuda")
     torch.cuda.synchronize()
     first = 0
-    for k in range(4):
-        cnt = (1 << 20) + (3 if k == 3 else 0)
+    for cnt in counts:
         engine.bond_curve_moments(hw.Rng(99, cnt, first_path=first), part.data_ptr())
         engine.synchronize()
         acc += part
+        torch.cuda.synchronize()
         first += cnt
     assert torch.allclose(full[1:101], acc[1:101], rtol=2e-8, atol=0)
     assert torch.allclose(full[102:], acc[102:], rtol=2e-7, atol=0)
@@ -403,11 +408,11 @@ def test_grid_stride_chunks_large_run(engine, hw, curve):
     torch.cuda.synchronize()
     engine.zbc_cv_moments(hw.Rng(99, n), curve["P"], curve["f"], zf.data_ptr(), n_steps_S1=500)
     first = 0
-    for k in range(4):
-        cnt = (1 << 20) + (3 if k == 3 else 0)
+    for cnt in counts:
         engine.zbc_cv_moments(hw.Rng(99, cnt, first_path=first), curve["P"], curve["f"], zp.data_ptr(), n_steps_S1=500)
         engine.synchronize()
         za += zp
+        torch.cuda.synchronize()
         first += cnt
     assert torch.allclose(zf, za, rtol=1e-12, atol=0)
 
