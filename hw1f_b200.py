@@ -16,6 +16,7 @@ Rng = _pkg.Rng
 HW1FError = _pkg.HW1FError
 default_params = _pkg.default_params
 caplet_schedule = _pkg.caplet_schedule
+swaption_schedule = _pkg.swaption_schedule
 Params = _pkg.Params
 LIB_PATH = _pkg.LIB_PATH
 _ffi = _pkg._ffi

@@ -305,6 +305,59 @@ int hw1f_cap_floor_moments(hw1f_engine* eng, hw1f_rng* rng, int32_t kind, const 
 int hw1f_cap_floor_finish(hw1f_engine* eng, const double* d_moments, uint64_t n_paths_total, const hw1f_caplet* caplets,
                           int32_t n_caplets, const float* P_mkt, hw1f_cap_result* out);
 
+/* ---- European swaptions: a book of coupon-bond options in one simulation pass ------------ */
+/* No reference call site.  A coupon-bond option pays, at its exercise date T_e,
+ *     N max(0, s (sum_j c_j P(T_e, T_j) - K)),   s = -1 payer (a put on the bond), +1 receiver (a call),
+ * over its cash flows (T_j, c_j).  A swaption on a swap starting at T_e with fixed rate kappa, accruals tau_j and notional
+ * M is the option with K = 1, c_j = kappa tau_j, c_last += 1 and N = M (the Python layer's swaption_schedule() builds
+ * them).  One launch prices every option of the book on one set of paths, each read at its exercise step, and returns
+ * the moments of each option and of the whole book, in both arithmetic modes and at any normal offset.  Payer and
+ * receiver options may be mixed in one book. */
+typedef struct hw1f_cash_flow {
+    float T;                /* payment date, T_exercise < T <= T_final, strictly increasing within an option */
+    float c;                /* amount per unit of N (> 0) */
+} hw1f_cash_flow;
+
+typedef struct hw1f_swaption {
+    float T_exercise;       /* exercise date (> 0), on the step grid like T_reset of hw1f_caplet              */
+    float K;                /* coupon-bond strike (> 0): 1 for a swap starting at T_exercise                   */
+    float N;                /* multiplier (> 0)                                                                */
+    int32_t kind;           /* HW1F_KIND_PAYER (put on the coupon bond) or HW1F_KIND_RECEIVER (call)          */
+    int32_t n_steps_exercise;   /* step at which r is read; < 0: the step nearest to T_exercise / dt          */
+    int32_t first_flow, n_flows;    /* this option's cash flows: flows[first_flow, first_flow + n_flows)     */
+    int32_t reserved;
+} hw1f_swaption;
+
+#define HW1F_KIND_PAYER 0
+#define HW1F_KIND_RECEIVER 1
+#define HW1F_MAX_SWAPTIONS 100        /* 5 (100 + 1) = 505 doubles: fits the peer mailboxes, as for caps          */
+#define HW1F_MAX_SWAPTION_FLOWS 2048  /* sum of n_flows over the book (a flow two options share counts twice):
+                                       * the per-flow bond plans live in the kernel's shared memory                  */
+
+/* Exercise steps round to the nearest step, as reset steps do for caplets.  The options must come in non-decreasing
+ * exercise steps; several may share a step (an expiry x tenor grid).
+ * Every argument is checked before any launch; HW1F_ERR_INVALID (with a message) for: a kind other than HW1F_KIND_PAYER /
+ * HW1F_KIND_RECEIVER, n_swaptions outside [1, HW1F_MAX_SWAPTIONS], n_flows (the length of `flows`) < 1 or the sum of the
+ * options' n_flows outside [1, HW1F_MAX_SWAPTION_FLOWS], an option's n_flows < 1 or a flow range outside `flows`, flow
+ * dates not strictly increasing or with the first <= T_exercise or the last > T_final, c, K or N not finite and
+ * positive (a forward-starting swap, whose first flow is negative, is out of scope), T_exercise off the step grid, an
+ * exercise step outside [1, n_steps] or exercise steps that decrease along the book.  After a failure the rng has not
+ * moved and no kernel was launched.
+ * Moments and statistics follow hw1f_cap_result (antithetic pairs); the control of an option is
+ * Y = N D(T_e) sum_j c_j P(T_e, T_j), whose known mean is N sum_j c_j P_mkt(T_j) (interpolated like interp_mkt).  The
+ * book's price uses ONE beta on Y_book = sum_i Y_i. */
+/* out[n_swaptions + 1]: the options in order, then the book.  Advances rng by the last exercise step. */
+int hw1f_swaptions(hw1f_engine* eng, hw1f_rng* rng, const hw1f_swaption* swaptions, int32_t n_swaptions,
+                   const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
+                   hw1f_cap_result* out, float* sim_ms);
+/* split form: d_moments[5 (n_swaptions + 1)] on the device; honours hw1f_comm_attach */
+int hw1f_swaptions_moments(hw1f_engine* eng, hw1f_rng* rng, const hw1f_swaption* swaptions, int32_t n_swaptions,
+                           const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
+                           double* d_moments);
+int hw1f_swaptions_finish(hw1f_engine* eng, const double* d_moments, uint64_t n_paths_total,
+                          const hw1f_swaption* swaptions, int32_t n_swaptions, const hw1f_cash_flow* flows,
+                          int32_t n_flows, const float* P_mkt, hw1f_cap_result* out);
+
 /* ---- fused pass (BASELINE.json scaling run) --------------------------------------------- */
 /* One launch: antithetic curve sums on the maturity grid + ZBC/control moments + pathwise-vega
  * tangent (both antithetic twins) evaluated at step n_steps_S1, all on the same normals.

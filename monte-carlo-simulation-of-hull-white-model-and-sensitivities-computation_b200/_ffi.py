@@ -13,6 +13,9 @@ ASYNC_SLOTS = 4   # HW1F_ASYNC_SLOTS
 ERR_INVALID, ERR_CUDA, ERR_NO_DEVICE, ERR_UNSUPPORTED, ERR_NO_MODEL, ERR_COMM = 1, 2, 3, 4, 5, 6
 KIND_CAP, KIND_FLOOR = 0, 1   # HW1F_KIND_*
 MAX_CAPLETS = 100             # HW1F_MAX_CAPLETS
+KIND_PAYER, KIND_RECEIVER = 0, 1   # HW1F_KIND_PAYER / HW1F_KIND_RECEIVER
+MAX_SWAPTIONS = 100                # HW1F_MAX_SWAPTIONS
+MAX_SWAPTION_FLOWS = 2048          # HW1F_MAX_SWAPTION_FLOWS
 
 
 class Params(C.Structure):
@@ -77,6 +80,18 @@ class CapResult(C.Structure):
         return d
 
 
+class CashFlow(C.Structure):
+    """hw1f_cash_flow: one payment (T, c) of a coupon bond."""
+    _fields_ = [("T", C.c_float), ("c", C.c_float)]
+
+
+class Swaption(C.Structure):
+    """hw1f_swaption: an option on the coupon bond flows[first_flow, first_flow + n_flows), exercised at T_exercise."""
+    _fields_ = [("T_exercise", C.c_float), ("K", C.c_float), ("N", C.c_float), ("kind", C.c_int32),
+                ("n_steps_exercise", C.c_int32), ("first_flow", C.c_int32), ("n_flows", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
 # every symbol include/hw1f.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _F = C.POINTER(C.c_float)
@@ -130,6 +145,9 @@ SYMBOLS = {
     "hw1f_cap_floor": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.POINTER(CapResult), _F]),
     "hw1f_cap_floor_moments": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "hw1f_cap_floor_finish": (C.c_int, [_P, _P, C.c_uint64, _P, C.c_int32, _P, C.POINTER(CapResult)]),
+    "hw1f_swaptions": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.POINTER(CapResult), _F]),
+    "hw1f_swaptions_moments": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
+    "hw1f_swaptions_finish": (C.c_int, [_P, _P, C.c_uint64, _P, C.c_int32, _P, C.c_int32, _P, C.POINTER(CapResult)]),
     "hw1f_fused_moments": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_int32, _P]),
     "hw1f_fused_fd_moments": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_float, C.c_int32, _P]),
     "hw1f_fused": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_float, C.c_int32, _P, _P, _P,

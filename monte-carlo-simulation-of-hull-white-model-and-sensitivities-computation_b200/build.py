@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libhw1f.so")
 SOURCES = ["hw1f_api.cu", "hw1f_multi.cu", "hw1f_comm.cu", "xorwow_jump.cpp"]
-HEADERS = ["hw1f_kernels.cuh", "hw1f_device.cuh", "hw1f_probe.cuh", "hw1f_kernels_extra.cuh", "hw1f_kernels_fast.cuh", "hw1f_kernels_cap.cuh", "hw1f_tail.cuh", "hw1f_comm.cuh", "xorwow_jump.hpp", os.path.join("..", "..", "include", "hw1f.h")]
+HEADERS = ["hw1f_kernels.cuh", "hw1f_device.cuh", "hw1f_probe.cuh", "hw1f_kernels_extra.cuh", "hw1f_kernels_fast.cuh", "hw1f_kernels_cap.cuh", "hw1f_kernels_swaption.cuh", "hw1f_tail.cuh", "hw1f_comm.cuh", "xorwow_jump.hpp", os.path.join("..", "..", "include", "hw1f.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -20,6 +20,7 @@
 #include "hw1f_kernels_extra.cuh"
 #include "hw1f_kernels_fast.cuh"
 #include "hw1f_kernels_cap.cuh"
+#include "hw1f_kernels_swaption.cuh"
 #include "hw1f_tail.cuh"
 #include "hw1f_probe.cuh"
 #include "xorwow_jump.hpp"
@@ -107,7 +108,7 @@ struct hw1f_engine {
     DevBuf<float2> d_state;              // dumped noise state (h, q) per subsequence (recalibrated FD, one pass)
     DevBuf<double> d_moments;            // internal moment vector
     DevBuf<float> d_out;                 // epilogue outputs
-    DevBuf<char> d_cap;                  // hw1f_cap_floor*: caplet table + market curves, one staged upload per call
+    DevBuf<char> d_cap;                  // hw1f_cap_floor* / hw1f_swaptions*: product tables + market curves, one staged upload per call
     DevBuf<int> d_int;
     void* h_stage = nullptr;             // pinned
     size_t h_stage_bytes = 0;
@@ -974,6 +975,8 @@ int init_kernels(hw1f_engine* e)
     HW_CUDA(e, opt_in(zbc_sum_kernel<3>, b));
     HW_CUDA(e, opt_in(cap_kernel<0>, b));
     HW_CUDA(e, opt_in(cap_kernel<1>, b));
+    HW_CUDA(e, opt_in(swaption_kernel<0>, b));
+    HW_CUDA(e, opt_in(swaption_kernel<1>, b));
     // the small kernels have no dynamic shared memory; querying them loads their code now instead
     // of inside the first timed call
     cudaFuncAttributes attr;
@@ -2376,6 +2379,179 @@ int hw1f_cap_floor(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caple
     std::vector<double> mom(res_mom(e, 0), res_mom(e, 0) + nq);
     HW_TRY(require_finite(e, mom.data(), (int)nq));
     cap_results(e, mom.data(), rng->n_paths, caps, n, P_mkt, out);
+    if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
+    return HW1F_OK;
+}
+
+// ---- European swaptions -------------------------------------------------------------------------
+static_assert(kMaxSwaptions == HW1F_MAX_SWAPTIONS && kMaxSwaptionFlows == HW1F_MAX_SWAPTION_FLOWS, "limits of hw1f.h");
+static_assert(sizeof(hw1f_swaption) == 32 && sizeof(hw1f_cash_flow) == 8, "ABI structs of hw1f.h");
+// every argument checked before any launch; steps[i] = the resolved exercise step of option i, *n_rows = sum of n_flows
+static int swaption_validate(hw1f_engine* e, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                             int32_t n_flows, std::vector<int>& steps, int* n_rows)
+{
+    HW_REQUIRE(e, n >= 1 && n <= HW1F_MAX_SWAPTIONS, "n_swaptions must be in [1, HW1F_MAX_SWAPTIONS]");
+    HW_REQUIRE(e, n_flows >= 1, "n_flows must be >= 1");
+    steps.assign(n, 0);
+    const double dt = (double)e->dt;
+    long rows = 0;
+    for (int i = 0; i < n; ++i) {
+        const hw1f_swaption& s = sw[i];
+        const std::string at = " (swaption " + std::to_string(i) + ")";
+        HW_REQUIRE(e, s.kind == HW1F_KIND_PAYER || s.kind == HW1F_KIND_RECEIVER,
+                   "kind must be HW1F_KIND_PAYER or HW1F_KIND_RECEIVER" + at);
+        HW_REQUIRE(e, std::isfinite(s.T_exercise) && s.T_exercise > 0.0f, "T_exercise must be finite and positive" + at);
+        HW_REQUIRE(e, std::isfinite(s.K) && s.K > 0.0f, "K must be finite and positive" + at);
+        HW_REQUIRE(e, std::isfinite(s.N) && s.N > 0.0f, "N must be finite and positive" + at);
+        HW_REQUIRE(e, s.n_flows >= 1, "n_flows of a swaption must be >= 1" + at);
+        HW_REQUIRE(e, s.first_flow >= 0 && (long)s.first_flow + s.n_flows <= n_flows, "flow range outside flows" + at);
+        rows += s.n_flows;
+        HW_REQUIRE(e, rows <= HW1F_MAX_SWAPTION_FLOWS, "the book's flows exceed HW1F_MAX_SWAPTION_FLOWS" + at);
+        float prev = s.T_exercise;
+        for (int j = s.first_flow; j < s.first_flow + s.n_flows; ++j) {
+            const hw1f_cash_flow& f = flows[j];
+            const std::string fat = " (swaption " + std::to_string(i) + ", flow " + std::to_string(j) + ")";
+            HW_REQUIRE(e, std::isfinite(f.T) && f.T > prev,
+                       "flow dates must be strictly increasing and after T_exercise" + fat);
+            HW_REQUIRE(e, std::isfinite(f.c) && f.c > 0.0f, "c must be finite and positive" + fat);
+            prev = f.T;
+        }
+        HW_REQUIRE(e, prev <= e->p.T_final, "the last flow date must not exceed T_final" + at);
+        long k = s.n_steps_exercise;
+        if (k < 0) {
+            k = std::lround((double)s.T_exercise / dt);
+            HW_REQUIRE(e, std::fabs((double)s.T_exercise - (double)k * dt) <= 1e-3 * dt,
+                       "T_exercise is not on the step grid (|T_exercise - k dt| > 1e-3 dt): pass n_steps_exercise" + at);
+        }
+        HW_REQUIRE(e, k >= 1 && k <= e->p.n_steps, "exercise step outside [1, n_steps]" + at);
+        HW_REQUIRE(e, i == 0 || k >= steps[i - 1], "exercise steps must be non-decreasing along the book" + at);
+        steps[i] = (int)k;
+    }
+    *n_rows = (int)rows;
+    return HW1F_OK;
+}
+
+// one staged upload of [option table | flow table | P_mkt | f_mkt], the launch and its tail.  The flow table holds each
+// option's flows in its own contiguous rows, with its exercise date beside them.
+static int swaption_run(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                        const std::vector<int>& steps, int n_rows, const float* P_mkt, const float* f_mkt,
+                        double* d_moments, const Finish& fin)
+{
+    const int nm = e->p.n_mat, nq = 5 * (n + 1);
+    const size_t tab = ((size_t)n * sizeof(SwaptionDev) + 255) & ~(size_t)255;
+    const size_t ftab = ((size_t)n_rows * sizeof(SwFlowDev) + 255) & ~(size_t)255;
+    std::vector<char> h(tab + ftab + 2 * (size_t)nm * sizeof(float), 0);
+    SwaptionDev* sd = reinterpret_cast<SwaptionDev*>(h.data());
+    SwFlowDev* fd = reinterpret_cast<SwFlowDev*>(h.data() + tab);
+    int row = 0;
+    for (int i = 0; i < n; ++i) {
+        sd[i].T_e = sw[i].T_exercise;
+        sd[i].K = sw[i].K;
+        sd[i].N = sw[i].N;
+        sd[i].sgn = (sw[i].kind == HW1F_KIND_PAYER) ? -1.0f : 1.0f;
+        sd[i].m = (float)e->det_m[0][steps[i]];
+        sd[i].Im = (float)e->det_I[0][steps[i]];
+        sd[i].step = steps[i];
+        sd[i].f0 = row;
+        sd[i].nf = sw[i].n_flows;
+        for (int j = 0; j < sw[i].n_flows; ++j, ++row) {
+            fd[row].T_e = sw[i].T_exercise;
+            fd[row].T = flows[sw[i].first_flow + j].T;
+            fd[row].c = flows[sw[i].first_flow + j].c;
+        }
+    }
+    memcpy(h.data() + tab + ftab, P_mkt, nm * sizeof(float));
+    memcpy(h.data() + tab + ftab + nm * sizeof(float), f_mkt, nm * sizeof(float));
+    const int decomp = e->mode == HW1F_MODE_DECOMPOSED;
+    const size_t smem = swaption_smem_bytes(decomp, n, n_rows, steps[n - 1]);
+    HW_TRY(decomp ? set_smem(e, swaption_kernel<1>, smem) : set_smem(e, swaption_kernel<0>, smem));
+    HW_CUDA(e, e->d_cap.ensure(h.size()));
+    HW_TRY(upload(e, e->d_cap.p, h.data(), h.size()));
+    Launch L;
+    HW_TRY(prepare_launch(e, &rng->seed, 1, rng->first_path, rng->n_paths, rng->offset, &L));
+    HW_CUDA(e, e->d_partials.ensure((size_t)L.grid_x * nq));
+    const ScenDev sc = scen_dev(e, e->p.sigma, e->sig_st, 0);
+    const SwaptionDev* d_sw = reinterpret_cast<const SwaptionDev*>(e->d_cap.p);
+    const SwFlowDev* d_fl = reinterpret_cast<const SwFlowDev*>(e->d_cap.p + tab);
+    const float* d_P = reinterpret_cast<const float*>(e->d_cap.p + tab + ftab);
+    HW_CUDA(e, launch_k(decomp ? swaption_kernel<1> : swaption_kernel<0>, dim3(L.grid_x, 1), kThreads, smem, e->stream,
+                        true, L.g, L.seeds, model_dev(e), sc, d_sw, (int)n, d_fl, n_rows, d_P, d_P + nm, L.lead,
+                        e->d_partials.p));
+    HW_TRY(check_launch(e, "swaption_kernel"));
+    HW_TRY(launch_tail(e, L, L.g.n_paths, nq, 0, nullptr, nullptr, 0.f, d_moments, nq, nq, fin));
+    rng->offset += (uint64_t)steps[n - 1];
+    return HW1F_OK;
+}
+
+static void swaption_results(const hw1f_engine* e, const double* mom, uint64_t n_pairs, const hw1f_swaption* sw,
+                             int32_t n, const hw1f_cash_flow* flows, const float* P_mkt, hw1f_cap_result* out)
+{
+    double book_mean = 0.0;
+    for (int i = 0; i < n; ++i) {
+        double annuity = 0.0;
+        for (int j = sw[i].first_flow; j < sw[i].first_flow + sw[i].n_flows; ++j)
+            annuity += (double)flows[j].c * (double)host_interp_mkt(e, P_mkt, flows[j].T);
+        const double cm = (double)sw[i].N * annuity;
+        book_mean += cm;
+        cap_algebra(mom + 5 * i, n_pairs, cm, out + i);
+    }
+    cap_algebra(mom + 5 * n, n_pairs, book_mean, out + n);
+}
+
+int hw1f_swaptions_moments(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n,
+                           const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
+                           double* d_moments)
+{
+    HW_TRY(require_model(e));
+    if (!rng || !sw || !flows || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    int rows = 0;
+    HW_TRY(swaption_validate(e, sw, n, flows, n_flows, steps, &rows));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    Finish fin;
+    fin.exchange = true;   // with peers attached (hw1f_comm_attach) the last block all-reduces the vector itself
+    return swaption_run(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, d_moments, fin);
+}
+
+int hw1f_swaptions_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths_total, const hw1f_swaption* sw,
+                          int32_t n, const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt,
+                          hw1f_cap_result* out)
+{
+    HW_TRY(require_model(e));
+    if (!d_moments || !sw || !flows || !P_mkt || !out) return HW1F_ERR_INVALID;
+    HW_REQUIRE(e, n_paths_total >= 1 && n_paths_total < (1ull << 40), "n_paths_total outside [1, 2^40)");
+    std::vector<int> steps;
+    int rows = 0;
+    HW_TRY(swaption_validate(e, sw, n, flows, n_flows, steps, &rows));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    std::vector<double> mom(5 * (size_t)(n + 1));
+    HW_TRY(download(e, mom.data(), d_moments, mom.size() * sizeof(double)));
+    HW_TRY(require_finite(e, mom.data(), (int)mom.size()));
+    swaption_results(e, mom.data(), n_paths_total, sw, n, flows, P_mkt, out);
+    return HW1F_OK;
+}
+
+int hw1f_swaptions(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                   int32_t n_flows, const float* P_mkt, const float* f_mkt, hw1f_cap_result* out, float* sim_ms)
+{
+    HW_TRY(require_model(e));
+    if (!rng || !sw || !flows || !P_mkt || !f_mkt || !out) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    int rows = 0;
+    HW_TRY(swaption_validate(e, sw, n, flows, n_flows, steps, &rows));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    const size_t nq = 5 * (size_t)(n + 1);
+    HW_CUDA(e, e->d_moments.ensure(std::max(4 * (size_t)e->p.n_mat * kMaxRuns, nq)));
+    HW_TRY(warm_geometry(e, rng));
+    Finish fin;
+    fin.host_mom = res_mom(e, 0);   // the result area holds at least 512 doubles
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev0, e->stream));
+    HW_TRY(swaption_run(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, e->d_moments.p, fin));
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev1, e->stream));
+    HW_TRY(wait_results(e));
+    std::vector<double> mom(res_mom(e, 0), res_mom(e, 0) + nq);
+    HW_TRY(require_finite(e, mom.data(), (int)nq));
+    swaption_results(e, mom.data(), rng->n_paths, sw, n, flows, P_mkt, out);
     if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
     return HW1F_OK;
 }

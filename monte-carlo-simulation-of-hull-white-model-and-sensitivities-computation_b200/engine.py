@@ -8,7 +8,7 @@ import ctypes as C
 import numpy as np
 
 from . import _ffi
-from ._ffi import CapResult, Caplet, Constants, Params, VegaResult, ZbcResult
+from ._ffi import CapResult, Caplet, CashFlow, Constants, Params, Swaption, VegaResult, ZbcResult
 
 
 class HW1FError(RuntimeError):
@@ -98,6 +98,72 @@ def _cap_results(res, n):
            for k in ("price_cv", "se_cv", "price_raw", "se_raw", "beta", "corr", "control_mean")}
     out["mom"] = np.array([r["mom"] for r in rows], np.float64).reshape(n, 5)
     out["strip"] = res[n].as_dict()
+    return out
+
+
+# numpy mirrors of hw1f_swaption and hw1f_cash_flow
+SWAPTION_DTYPE = np.dtype([(n, np.float32 if t is C.c_float else np.int32) for n, t in Swaption._fields_])
+CASH_FLOW_DTYPE = np.dtype([(n, np.float32) for n, _ in CashFlow._fields_])
+assert SWAPTION_DTYPE.itemsize == C.sizeof(Swaption) and CASH_FLOW_DTYPE.itemsize == C.sizeof(CashFlow)
+
+
+def _swaption_kind(kind):
+    if kind in ("payer", _ffi.KIND_PAYER):
+        return _ffi.KIND_PAYER
+    if kind in ("receiver", _ffi.KIND_RECEIVER):
+        return _ffi.KIND_RECEIVER
+    return int(kind) if isinstance(kind, (int, np.integer)) else -1   # the engine rejects it with a message
+
+
+def swaption_schedule(expiries, tenors, strike_rate, freq=1, notional=1.0, kind="payer"):
+    """European swaptions on spot-starting swaps, one per (expiry, tenor) pair (the arguments broadcast against each
+    other; a grid is expiries and tenors repeated to its cells), as the coupon-bond options the engine prices.  The
+    swap from T_e to T_e + tenor pays the fixed rate kappa every 1 / freq years, so the option is on the bond with flows
+    c = kappa / freq at T_e + k / freq (the last c += 1), strike K = 1 and multiplier N = M (notional); a payer
+    swaption is a put on that bond, a receiver swaption a call.  Exercise steps are left to the engine
+    (n_steps_exercise = -1: the step nearest to T_e / dt).  Returns (swaptions, flows), structured arrays of
+    hw1f_swaption and hw1f_cash_flow; no GPU needed."""
+    kinds = np.asarray(kind, dtype=object)
+    Te, ten, kappa, M, kd = np.broadcast_arrays(np.asarray(expiries, np.float64), np.asarray(tenors, np.float64),
+                                                np.asarray(strike_rate, np.float64), np.asarray(notional, np.float64),
+                                                kinds)
+    Te, ten, kappa, M, kd = (np.atleast_1d(a).ravel() for a in (Te, ten, kappa, M, kd))
+    n_cpn = np.rint(ten * freq).astype(np.int64)
+    if (n_cpn < 1).any() or (np.abs(ten * freq - n_cpn) > 1e-9).any():
+        raise ValueError("every tenor must be a positive whole number of coupon periods (tenor * freq)")
+    sw = np.zeros(len(Te), SWAPTION_DTYPE)
+    fl = np.zeros(int(n_cpn.sum()), CASH_FLOW_DTYPE)
+    row = 0
+    for i in range(len(Te)):
+        k = np.arange(1, n_cpn[i] + 1)
+        c = np.full(n_cpn[i], kappa[i] / freq)
+        c[-1] += 1.0
+        fl["T"][row:row + n_cpn[i]] = Te[i] + k / freq
+        fl["c"][row:row + n_cpn[i]] = c
+        sw[i] = (Te[i], 1.0, M[i], _swaption_kind(kd[i]), -1, row, n_cpn[i], 0)
+        row += n_cpn[i]
+    return sw, fl
+
+
+def _swaption_book(swaptions, flows):
+    """structured arrays (swaption_schedule) or sequences of tuples in the field order of hw1f_swaption /
+    hw1f_cash_flow -> contiguous arrays of the ABI structs"""
+    def conv(x, dt, defaults):
+        if isinstance(x, np.ndarray) and x.dtype.names:
+            a = np.zeros(x.shape, dt)
+            for n in dt.names:
+                if n in x.dtype.names:
+                    a[n] = x[n]
+                elif n in defaults:
+                    a[n] = defaults[n]
+            return np.ascontiguousarray(a.ravel())
+        return np.array([tuple(r) for r in x], dt)
+    return conv(swaptions, SWAPTION_DTYPE, {"n_steps_exercise": -1}), conv(flows, CASH_FLOW_DTYPE, {})
+
+
+def _book_results(res, n):
+    out = _cap_results(res, n)
+    out["book"] = out.pop("strip")
     return out
 
 
@@ -349,6 +415,34 @@ class Engine:
         self._check(self._lib.hw1f_cap_floor_finish(self._h, C.c_void_p(d_moments_ptr), int(n_paths_total), _ptr(cap),
                                                     len(cap), _ptr(P_mkt), res))
         return _cap_results(res, len(cap))
+
+    # -- European swaptions: a book of coupon-bond options in one simulation pass (no reference call site) --
+    def swaptions(self, rng, swaptions, flows, P_mkt, f_mkt):
+        """swaptions, flows as from swaption_schedule().  Per-option arrays price_cv, se_cv, price_raw, se_raw, beta,
+        corr, control_mean, mom[n, 5], the whole book under "book", and sim_ms."""
+        sw, fl = _swaption_book(swaptions, flows)
+        P_mkt, f_mkt = _f32(P_mkt, self.n_mat), _f32(f_mkt, self.n_mat)
+        res, ms = (CapResult * (len(sw) + 1))(), C.c_float()
+        self._check(self._lib.hw1f_swaptions(self._h, rng._h, _ptr(sw), len(sw), _ptr(fl), len(fl), _ptr(P_mkt),
+                                             _ptr(f_mkt), res, C.byref(ms)))
+        out = _book_results(res, len(sw))
+        out["sim_ms"] = ms.value
+        return out
+
+    def swaptions_moments(self, rng, swaptions, flows, P_mkt, f_mkt, d_moments_ptr):
+        """async: device pointer to 5 * (len(swaptions) + 1) doubles"""
+        sw, fl = _swaption_book(swaptions, flows)
+        P_mkt, f_mkt = _f32(P_mkt, self.n_mat), _f32(f_mkt, self.n_mat)
+        self._check(self._lib.hw1f_swaptions_moments(self._h, rng._h, _ptr(sw), len(sw), _ptr(fl), len(fl),
+                                                     _ptr(P_mkt), _ptr(f_mkt), C.c_void_p(d_moments_ptr)))
+
+    def swaptions_finish(self, d_moments_ptr, n_paths_total, swaptions, flows, P_mkt):
+        sw, fl = _swaption_book(swaptions, flows)
+        P_mkt = _f32(P_mkt, self.n_mat)
+        res = (CapResult * (len(sw) + 1))()
+        self._check(self._lib.hw1f_swaptions_finish(self._h, C.c_void_p(d_moments_ptr), int(n_paths_total), _ptr(sw),
+                                                    len(sw), _ptr(fl), len(fl), _ptr(P_mkt), res))
+        return _book_results(res, len(sw))
 
     # -- Q3 (src/3_sensitivity_analysis.cu) --
     def vega_pathwise(self, rng, P_mkt, f_mkt, S1=5.0, S2=10.0, K=None, n_steps_S1=-1):
