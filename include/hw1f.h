@@ -358,6 +358,49 @@ int hw1f_swaptions_finish(hw1f_engine* eng, const double* d_moments, uint64_t n_
                           const hw1f_swaption* swaptions, int32_t n_swaptions, const hw1f_cash_flow* flows,
                           int32_t n_flows, const float* P_mkt, hw1f_cap_result* out);
 
+/* ---- vega of a swaption book (or a cap strip): both sigma bumps on common random numbers -- */
+/* No reference call site.  The estimator of hw1f_vega_fd (run_finite_difference, src/3:400-446) for a whole book: one
+ * launch prices the book of hw1f_swaptions in three sigma scenarios -- sigma, sigma - eps, sigma + eps -- on ONE set of
+ * normals, every path stepped once to the last exercise step.  In decomposed mode the bumped scenarios share the noise
+ * recursion of the base one and add only their payoffs at the exercise steps.
+ *   * The base scenario performs the float operations of hw1f_swaptions: out[] is bit-identical to what hw1f_swaptions
+ *     returns for the same arguments, and the rng advances the same.
+ *   * Each bumped model keeps the market curve: its drift is the shifted drift table of sigma -/+ eps built from the
+ *     model's own theta_a1 (fd_theta_a1, the reference's quirk for hw1f_vega_fd, is NOT read), its bond plans
+ *     P(T_e, T_j) = A(sigma -/+ eps) exp(-B r) are priced on the same P_mkt, f_mkt.
+ *   * The bumped prices are raw pair means, with no control variate (a control's known mean would be only as good as
+ *     the refit); vega_se says what that costs.
+ *   * Per antithetic pair X_s = N (x_s(+G) + x_s(-G)) and D = X_+ - X_-; the book's X_s and D are the sums over its
+ *     options.  vega = sum D / (2 n_pairs) / (2 eps), vega_se = sqrt(var(D / 2) / n_pairs) / (2 eps).
+ * Validation: everything hw1f_swaptions checks, plus eps finite with 0 < eps < sigma, and (split form with peers
+ * attached) 11 (n_swaptions + 1) <= 512 moments, the peer mailboxes, i.e. n_swaptions <= 45; larger books go through
+ * an external all-reduce and hw1f_swaptions_vega_finish.  After a failure (HW1F_ERR_INVALID with a message) the rng has
+ * not moved and no kernel was launched.  The kernel keeps the flow plans of three scenarios and, in reference order,
+ * three drift tables in shared memory: a book too large for it returns HW1F_ERR_UNSUPPORTED ("book too large for
+ * shared memory") before any launch, rng unmoved.  Decomposed mode prices every book validation accepts at the default
+ * 1000 steps.  Cap strips: a caplet is the one-flow option (c = 1, payer for a cap, receiver for a floor). */
+typedef struct hw1f_book_vega {      /* one option, or the whole book */
+    double mom[6];                   /* sum X-, X-^2, X+, X+^2, D, D^2 over antithetic pairs; D = X+ - X- */
+    double price_minus, se_minus;    /* raw pair-mean price at sigma - eps and its standard error */
+    double price_plus, se_plus;      /* the same at sigma + eps */
+    double vega, vega_se;            /* sum D / (2 n_pairs) / (2 eps);  sqrt(var(D / 2) / n_pairs) / (2 eps) */
+} hw1f_book_vega;
+
+/* out[n_swaptions + 1] as hw1f_swaptions (bit-identical), vega[n_swaptions + 1]: the options, then the book.
+ * Advances rng by the last exercise step. */
+int hw1f_swaptions_vega(hw1f_engine* eng, hw1f_rng* rng, const hw1f_swaption* swaptions, int32_t n_swaptions,
+                        const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt, float eps,
+                        hw1f_cap_result* out, hw1f_book_vega* vega, float* sim_ms);
+/* split form: d_moments[11 (n_swaptions + 1)] on the device -- [0, 5 (n + 1)) exactly the hw1f_swaptions_moments
+ * vector, then 6 per option (mom of hw1f_book_vega), then the book's 6; honours hw1f_comm_attach */
+int hw1f_swaptions_vega_moments(hw1f_engine* eng, hw1f_rng* rng, const hw1f_swaption* swaptions, int32_t n_swaptions,
+                                const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
+                                float eps, double* d_moments);
+int hw1f_swaptions_vega_finish(hw1f_engine* eng, const double* d_moments, uint64_t n_paths_total,
+                               const hw1f_swaption* swaptions, int32_t n_swaptions, const hw1f_cash_flow* flows,
+                               int32_t n_flows, const float* P_mkt, float eps, hw1f_cap_result* out,
+                               hw1f_book_vega* vega);
+
 /* ---- fused pass (BASELINE.json scaling run) --------------------------------------------- */
 /* One launch: antithetic curve sums on the maturity grid + ZBC/control moments + pathwise-vega
  * tangent (both antithetic twins) evaluated at step n_steps_S1, all on the same normals.

@@ -6,7 +6,7 @@ thin Python host layer over it.  There is no CPU fallback: importing works witho
 creating an Engine does not.
 """
 from . import _ffi, engine, parallel
-from ._ffi import LIB_PATH, CapResult, Caplet, CashFlow, Params, Swaption, VegaResult, ZbcResult
+from ._ffi import LIB_PATH, BookVega, CapResult, Caplet, CashFlow, Params, Swaption, VegaResult, ZbcResult
 from .engine import Engine, HW1FError, Rng, caplet_schedule, default_params, swaption_schedule
 
-__all__ = ["engine", "parallel", "Engine", "Rng", "HW1FError", "default_params", "caplet_schedule", "swaption_schedule", "Params", "Caplet", "CapResult", "Swaption", "CashFlow", "ZbcResult", "VegaResult", "LIB_PATH", "_ffi"]
+__all__ = ["engine", "parallel", "Engine", "Rng", "HW1FError", "default_params", "caplet_schedule", "swaption_schedule", "Params", "Caplet", "CapResult", "BookVega", "Swaption", "CashFlow", "ZbcResult", "VegaResult", "LIB_PATH", "_ffi"]

@@ -80,6 +80,17 @@ class CapResult(C.Structure):
         return d
 
 
+class BookVega(C.Structure):
+    """hw1f_book_vega: one option, or the whole book -- the sigma -/+ eps prices and the vega on common random numbers."""
+    _fields_ = [("mom", C.c_double * 6), ("price_minus", C.c_double), ("se_minus", C.c_double),
+                ("price_plus", C.c_double), ("se_plus", C.c_double), ("vega", C.c_double), ("vega_se", C.c_double)]
+
+    def as_dict(self):
+        d = {n: getattr(self, n) for n, _ in self._fields_ if n != "mom"}
+        d["mom"] = list(self.mom)
+        return d
+
+
 class CashFlow(C.Structure):
     """hw1f_cash_flow: one payment (T, c) of a coupon bond."""
     _fields_ = [("T", C.c_float), ("c", C.c_float)]
@@ -148,6 +159,11 @@ SYMBOLS = {
     "hw1f_swaptions": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.POINTER(CapResult), _F]),
     "hw1f_swaptions_moments": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, _P]),
     "hw1f_swaptions_finish": (C.c_int, [_P, _P, C.c_uint64, _P, C.c_int32, _P, C.c_int32, _P, C.POINTER(CapResult)]),
+    "hw1f_swaptions_vega": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_float, C.POINTER(CapResult),
+                                      C.POINTER(BookVega), _F]),
+    "hw1f_swaptions_vega_moments": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_float, _P]),
+    "hw1f_swaptions_vega_finish": (C.c_int, [_P, _P, C.c_uint64, _P, C.c_int32, _P, C.c_int32, _P, C.c_float,
+                                             C.POINTER(CapResult), C.POINTER(BookVega)]),
     "hw1f_fused_moments": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_int32, _P]),
     "hw1f_fused_fd_moments": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_float, C.c_int32, _P]),
     "hw1f_fused": (C.c_int, [_P, _P, C.c_float, C.c_float, C.c_float, _P, _P, C.c_float, C.c_int32, _P, _P, _P,

@@ -21,6 +21,7 @@
 #include "hw1f_kernels_fast.cuh"
 #include "hw1f_kernels_cap.cuh"
 #include "hw1f_kernels_swaption.cuh"
+#include "hw1f_kernels_book_vega.cuh"
 #include "hw1f_tail.cuh"
 #include "hw1f_probe.cuh"
 #include "xorwow_jump.hpp"
@@ -100,8 +101,9 @@ struct hw1f_engine {
     DevBuf<float> d_mkt;                 // [4][n_mat]: P0,f0,P1,f1
     DevBuf<float> d_center;              // [n_mat] centring constants of the curve accumulation
     // noise-free ("deterministic") parts per drift slot, host double: det_m[slot][i] = short rate
-    // after i steps with G = 0, det_I[slot][i] its trapezoid integral (slot 1: tangent D, ID)
-    std::vector<double> det_m[4], det_I[4];
+    // after i steps with G = 0, det_I[slot][i] its trapezoid integral (slot 1: tangent D, ID; slots 4, 5: the
+    // sigma -/+ eps scenarios of the book vega, see bv_*)
+    std::vector<double> det_m[6], det_I[6];
     DevBuf<float> d_emI[4];              // [n_mat] exp(-det_I) at the save points (decomposed curve kernels)
     DevBuf<BondPlan> d_plans;
     DevBuf<double> d_partials;
@@ -129,6 +131,12 @@ struct hw1f_engine {
     bool fd_cached = false;
     float fd_sig[2] = {0.f, 0.f};
     cudaEvent_t ev_fd = nullptr;
+    // book vega (hw1f_swaptions_vega*): shifted drift tables of sigma -/+ eps on the model's own theta_a1, and their
+    // noise-free tables in det slots 4, 5; host-side, rebuilt only when (model, sigma pair) changes.  Kept apart from
+    // the FD slots 2, 3, which hold hw1f_vega_fd's tables (fd_theta_a1)
+    bool bv_cached = false;
+    float bv_sig[2] = {0.f, 0.f};
+    std::vector<float> bv_drift[2];
     // tail of the simulation kernels (hw1f_tail.cuh): ticket counters, group partials, and the result areas in mapped
     // pinned host memory the last block stores into (the host only waits for the stream)
     DevBuf<unsigned> d_tail_cnt;
@@ -977,6 +985,8 @@ int init_kernels(hw1f_engine* e)
     HW_CUDA(e, opt_in(cap_kernel<1>, b));
     HW_CUDA(e, opt_in(swaption_kernel<0>, b));
     HW_CUDA(e, opt_in(swaption_kernel<1>, b));
+    HW_CUDA(e, opt_in(book_vega_kernel<0>, b));
+    HW_CUDA(e, opt_in(book_vega_kernel<1>, b));
     // the small kernels have no dynamic shared memory; querying them loads their code now instead
     // of inside the first timed call
     cudaFuncAttributes attr;
@@ -1242,6 +1252,7 @@ int hw1f_set_model(hw1f_engine* e, const hw1f_params* p)
         e->cached_p = *p;
         e->model_cached = true;
         e->fd_cached = false;      // the bumped-sigma tables and the step probe depend on the model
+        e->bv_cached = false;
         e->steps_cached = false;
     }
     {   // result areas: the longest moment vector (two curve scenarios + extras) and P, f, P_se of two curves
@@ -2552,6 +2563,240 @@ int hw1f_swaptions(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32
     std::vector<double> mom(res_mom(e, 0), res_mom(e, 0) + nq);
     HW_TRY(require_finite(e, mom.data(), (int)nq));
     swaption_results(e, mom.data(), rng->n_paths, sw, n, flows, P_mkt, out);
+    if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
+    return HW1F_OK;
+}
+
+// ---- vega of a swaption book: sigma -/+ eps on common random numbers in the pricing pass -----------------------
+static_assert(sizeof(hw1f_book_vega) == 12 * sizeof(double), "ABI struct of hw1f.h");
+
+// everything swaption_validate checks, and the bump
+static int book_vega_validate(hw1f_engine* e, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                              int32_t n_flows, float eps, std::vector<int>& steps, int* n_rows)
+{
+    HW_TRY(swaption_validate(e, sw, n, flows, n_flows, steps, n_rows));
+    HW_REQUIRE(e, std::isfinite(eps) && eps > 0.0f && eps < e->p.sigma, "eps must be finite with 0 < eps < sigma");
+    return HW1F_OK;
+}
+
+// the kernel's shared memory, checked before anything is launched or the rng moves
+static int book_vega_smem(hw1f_engine* e, int32_t n, int n_rows, const std::vector<int>& steps, size_t* smem)
+{
+    *smem = book_vega_smem_bytes(e->mode == HW1F_MODE_DECOMPOSED, n, n_rows, steps[n - 1]);
+    if (*smem + 2048 > e->smem_optin) {   // the head-room of set_smem
+        e->err = "book too large for shared memory (three scenarios' flow plans and, in reference order, drift tables: "
+                 "fewer flows, fewer steps, or decomposed mode)";
+        return HW1F_ERR_UNSUPPORTED;
+    }
+    return HW1F_OK;
+}
+
+// host tables of the bumped models: shifted drift tables of sigma -/+ eps on the model's own theta_a1 (fd_theta_a1 is
+// the reference's quirk for the ZBC of hw1f_vega_fd, which reads nothing after theta_break; a book may) and their
+// noise-free tables (det slots 4, 5).  Cached per (model, sigma pair), apart from hw1f_vega_fd's slots 2, 3.
+static void book_vega_tables(hw1f_engine* e, float sig_m, float sig_p)
+{
+    if (e->bv_cached && e->bv_sig[0] == sig_m && e->bv_sig[1] == sig_p) return;
+    hw1f_params q = e->p;
+    q.fd_theta_a1 = q.theta_a1;
+    for (int k = 0; k < 2; ++k) {
+        e->bv_drift[k].assign(e->p.n_steps, 0.f);
+        host_shifted_drift_table(q, k ? sig_p : sig_m, e->p.sigma, e->bv_drift[k].data());
+        build_det_tables(e, 4 + k, e->bv_drift[k].data(), nullptr);
+    }
+    e->bv_sig[0] = sig_m;
+    e->bv_sig[1] = sig_p;
+    e->bv_cached = true;
+}
+
+// tail_kernel (ncur = 0) over one of the launch's two partial-row sets; host_mom: null or the mapped result area
+static int book_vega_tail(hw1f_engine* e, const Launch& L, const double* partials, int nq, double* d_moments,
+                          double* host_mom, bool exchange)
+{
+    Finish fin;
+    fin.host_mom = host_mom;
+    fin.exchange = exchange;
+    TailArgs ta;
+    HW_TRY(make_tail(e, L.n_runs, L.grid_x, L.g.n_paths, nq, 0, nullptr, nullptr, 0.f, d_moments, nq, nq, fin, &ta));
+    const unsigned n_groups = (L.grid_x + kTailGroup - 1) / kTailGroup;
+    const size_t smem = tail_smem_bytes(nq, e->p.n_mat);
+    HW_REQUIRE(e, smem <= 48 * 1024, "moment vector too long for the tail kernel's shared memory");
+    HW_CUDA(e, launch_k(tail_kernel, dim3(n_groups, L.n_runs), dim3(kTailThreads), smem, e->stream, true, ta, model_dev(e),
+                        partials, (int)L.grid_x, nq, 0));
+    return check_launch(e, "tail_kernel");
+}
+
+// one staged upload of [option table | bumped noise-free tables | flow table | P_mkt | f_mkt | (reference order) two
+// shifted drift tables], the launch and the two tails: the base rows reduced as hw1f_swaptions reduces them (the tail
+// splits rows by the vector length, so one combined vector would sum them in another order), then the bumped rows.
+// host_mom: null or the mapped result area of 11 (n + 1) doubles.
+static int book_vega_run(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                         const std::vector<int>& steps, int n_rows, const float* P_mkt, const float* f_mkt, float eps,
+                         size_t smem, double* d_moments, double* host_mom, bool exchange)
+{
+    const int nm = e->p.n_mat, nb = 5 * (n + 1), nv = 6 * (n + 1), n_last = steps[n - 1];
+    const int decomp = e->mode == HW1F_MODE_DECOMPOSED;
+    const float sig_m = e->p.sigma - eps, sig_p = e->p.sigma + eps;
+    book_vega_tables(e, sig_m, sig_p);
+    auto align = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t tab = align((size_t)n * sizeof(SwaptionDev)), btab = align((size_t)n * sizeof(BookVegaOptDev));
+    const size_t ftab = align((size_t)n_rows * sizeof(SwFlowDev)), mtab = align(2 * (size_t)nm * sizeof(float));
+    const size_t dtab = decomp ? 0 : 2 * (size_t)n_last * sizeof(float);
+    std::vector<char> h(tab + btab + ftab + mtab + dtab, 0);
+    SwaptionDev* sd = reinterpret_cast<SwaptionDev*>(h.data());
+    BookVegaOptDev* bd = reinterpret_cast<BookVegaOptDev*>(h.data() + tab);
+    SwFlowDev* fd = reinterpret_cast<SwFlowDev*>(h.data() + tab + btab);
+    int row = 0;
+    for (int i = 0; i < n; ++i) {   // the option and flow tables of swaption_run
+        sd[i].T_e = sw[i].T_exercise;
+        sd[i].K = sw[i].K;
+        sd[i].N = sw[i].N;
+        sd[i].sgn = (sw[i].kind == HW1F_KIND_PAYER) ? -1.0f : 1.0f;
+        sd[i].m = (float)e->det_m[0][steps[i]];
+        sd[i].Im = (float)e->det_I[0][steps[i]];
+        sd[i].step = steps[i];
+        sd[i].f0 = row;
+        sd[i].nf = sw[i].n_flows;
+        for (int s = 0; s < 2; ++s) {
+            bd[i].m[s] = (float)e->det_m[4 + s][steps[i]];
+            bd[i].Im[s] = (float)e->det_I[4 + s][steps[i]];
+        }
+        for (int j = 0; j < sw[i].n_flows; ++j, ++row) {
+            fd[row].T_e = sw[i].T_exercise;
+            fd[row].T = flows[sw[i].first_flow + j].T;
+            fd[row].c = flows[sw[i].first_flow + j].c;
+        }
+    }
+    char* mkt = h.data() + tab + btab + ftab;
+    memcpy(mkt, P_mkt, nm * sizeof(float));
+    memcpy(mkt + nm * sizeof(float), f_mkt, nm * sizeof(float));
+    if (!decomp)
+        for (int s = 0; s < 2; ++s)
+            memcpy(mkt + mtab + (size_t)s * n_last * sizeof(float), e->bv_drift[s].data(), n_last * sizeof(float));
+    HW_CUDA(e, e->d_cap.ensure(h.size()));
+    HW_TRY(upload(e, e->d_cap.p, h.data(), h.size()));
+    Launch L;
+    HW_TRY(prepare_launch(e, &rng->seed, 1, rng->first_path, rng->n_paths, rng->offset, &L));
+    HW_CUDA(e, e->d_partials.ensure((size_t)L.grid_x * (nb + nv)));
+    const ScenDev sc = scen_dev(e, e->p.sigma, e->sig_st, 0);
+    BookVegaScen bv;
+    const float* d_mkt = reinterpret_cast<const float*>(e->d_cap.p + tab + btab + ftab);
+    for (int s = 0; s < 2; ++s) {
+        bv.sigma[s] = s ? sig_p : sig_m;
+        bv.sig_st[s] = host_sig_st(e->p, bv.sigma[s]);
+        bv.drift[s] = decomp ? nullptr : reinterpret_cast<const float*>(e->d_cap.p + tab + btab + ftab + mtab) + s * n_last;
+    }
+    const SwaptionDev* d_sw = reinterpret_cast<const SwaptionDev*>(e->d_cap.p);
+    const BookVegaOptDev* d_bo = reinterpret_cast<const BookVegaOptDev*>(e->d_cap.p + tab);
+    const SwFlowDev* d_fl = reinterpret_cast<const SwFlowDev*>(e->d_cap.p + tab + btab);
+    double* part_b = e->d_partials.p;
+    double* part_v = e->d_partials.p + (size_t)L.grid_x * nb;
+    HW_CUDA(e, launch_k(decomp ? book_vega_kernel<1> : book_vega_kernel<0>, dim3(L.grid_x, 1), kThreads, smem, e->stream,
+                        true, L.g, L.seeds, model_dev(e), sc, bv, d_sw, d_bo, (int)n, d_fl, n_rows, d_mkt, d_mkt + nm,
+                        L.lead, part_b, part_v));
+    HW_TRY(check_launch(e, "book_vega_kernel"));
+    HW_TRY(book_vega_tail(e, L, part_b, nb, d_moments, host_mom, exchange));
+    HW_TRY(book_vega_tail(e, L, part_v, nv, d_moments + nb, host_mom ? host_mom + nb : nullptr, exchange));
+    rng->offset += (uint64_t)n_last;
+    return HW1F_OK;
+}
+
+// pair-mean price and standard error of n_pairs samples x = X / 2 from (sum X, sum X^2)
+static void pair_mean(double sX, double sXX, uint64_t n_pairs, double* mean, double* se)
+{
+    const double n = (double)n_pairs, d = n > 1.0 ? n - 1.0 : 1.0;
+    const double sx = 0.5 * sX, sxx = 0.25 * sXX, mx = sx / n;
+    double v = (sxx - sx * mx) / d;
+    if (v < 0.0) v = 0.0;
+    *mean = mx;
+    *se = sqrt(v / n);
+}
+
+static void book_vega_results(const hw1f_engine* e, const double* mom, uint64_t n_pairs, const hw1f_swaption* sw,
+                              int32_t n, const hw1f_cash_flow* flows, const float* P_mkt, float eps, hw1f_cap_result* out,
+                              hw1f_book_vega* vega)
+{
+    swaption_results(e, mom, n_pairs, sw, n, flows, P_mkt, out);
+    const double h = 2.0 * (double)eps;
+    for (int i = 0; i <= n; ++i) {
+        const double* m = mom + 5 * (n + 1) + 6 * i;
+        hw1f_book_vega* v = vega + i;
+        memset(v, 0, sizeof(*v));
+        for (int k = 0; k < 6; ++k) v->mom[k] = m[k];
+        pair_mean(m[0], m[1], n_pairs, &v->price_minus, &v->se_minus);
+        pair_mean(m[2], m[3], n_pairs, &v->price_plus, &v->se_plus);
+        double d, d_se;
+        pair_mean(m[4], m[5], n_pairs, &d, &d_se);
+        v->vega = d / h;
+        v->vega_se = d_se / h;
+    }
+}
+
+int hw1f_swaptions_vega_moments(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n,
+                                const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
+                                float eps, double* d_moments)
+{
+    HW_TRY(require_model(e));
+    if (!rng || !sw || !flows || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    int rows = 0;
+    HW_TRY(book_vega_validate(e, sw, n, flows, n_flows, eps, steps, &rows));
+    // with peers attached the tails all-reduce the vector (hw1f_comm_attach); checked here, not after the launch
+    HW_REQUIRE(e, !e->comm_on || 11 * (n + 1) <= kCommMaxCount,
+               "with peers attached 11 (n_swaptions + 1) moments must fit the peer mailboxes (512): n_swaptions <= 45");
+    size_t smem = 0;
+    HW_TRY(book_vega_smem(e, n, rows, steps, &smem));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    return book_vega_run(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, eps, smem, d_moments, nullptr, true);
+}
+
+int hw1f_swaptions_vega_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths_total, const hw1f_swaption* sw,
+                               int32_t n, const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, float eps,
+                               hw1f_cap_result* out, hw1f_book_vega* vega)
+{
+    HW_TRY(require_model(e));
+    if (!d_moments || !sw || !flows || !P_mkt || !out || !vega) return HW1F_ERR_INVALID;
+    HW_REQUIRE(e, n_paths_total >= 1 && n_paths_total < (1ull << 40), "n_paths_total outside [1, 2^40)");
+    std::vector<int> steps;
+    int rows = 0;
+    HW_TRY(book_vega_validate(e, sw, n, flows, n_flows, eps, steps, &rows));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    std::vector<double> mom(11 * (size_t)(n + 1));
+    HW_TRY(download(e, mom.data(), d_moments, mom.size() * sizeof(double)));
+    HW_TRY(require_finite(e, mom.data(), (int)mom.size()));
+    book_vega_results(e, mom.data(), n_paths_total, sw, n, flows, P_mkt, eps, out, vega);
+    return HW1F_OK;
+}
+
+int hw1f_swaptions_vega(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                        int32_t n_flows, const float* P_mkt, const float* f_mkt, float eps, hw1f_cap_result* out,
+                        hw1f_book_vega* vega, float* sim_ms)
+{
+    HW_TRY(require_model(e));
+    if (!rng || !sw || !flows || !P_mkt || !f_mkt || !out || !vega) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    int rows = 0;
+    HW_TRY(book_vega_validate(e, sw, n, flows, n_flows, eps, steps, &rows));
+    size_t smem = 0;
+    HW_TRY(book_vega_smem(e, n, rows, steps, &smem));
+    HW_CUDA(e, cudaSetDevice(e->device));
+    const size_t nq = 11 * (size_t)(n + 1);
+    HW_CUDA(e, e->d_moments.ensure(std::max(4 * (size_t)e->p.n_mat * kMaxRuns, nq)));
+    HW_TRY(warm_geometry(e, rng));
+    // the mapped result area holds max(4 n_mat + 64, 512) doubles; a longer vector is read back from the device
+    double* host_mom = nq <= e->res_doubles ? res_mom(e, 0) : nullptr;
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev0, e->stream));
+    HW_TRY(book_vega_run(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, eps, smem, e->d_moments.p, host_mom, false));
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev1, e->stream));
+    std::vector<double> mom(nq);
+    if (host_mom) {
+        HW_TRY(wait_results(e));
+        memcpy(mom.data(), host_mom, nq * sizeof(double));
+    } else {
+        HW_TRY(download(e, mom.data(), e->d_moments.p, nq * sizeof(double)));
+    }
+    HW_TRY(require_finite(e, mom.data(), (int)nq));
+    book_vega_results(e, mom.data(), rng->n_paths, sw, n, flows, P_mkt, eps, out, vega);
     if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
     return HW1F_OK;
 }

@@ -8,7 +8,7 @@ import ctypes as C
 import numpy as np
 
 from . import _ffi
-from ._ffi import CapResult, Caplet, CashFlow, Constants, Params, Swaption, VegaResult, ZbcResult
+from ._ffi import BookVega, CapResult, Caplet, CashFlow, Constants, Params, Swaption, VegaResult, ZbcResult
 
 
 class HW1FError(RuntimeError):
@@ -165,6 +165,34 @@ def _book_results(res, n):
     out = _cap_results(res, n)
     out["book"] = out.pop("strip")
     return out
+
+
+def _add_vega(out, vres, n, book_key):
+    """the hw1f_book_vega rows into a result dict: per-option arrays, and the book's values into out[book_key]"""
+    rows = [vres[i].as_dict() for i in range(n)]
+    for k in ("price_minus", "se_minus", "price_plus", "se_plus", "vega", "vega_se"):
+        out[k] = np.array([r[k] for r in rows], np.float64)
+    out["vega_mom"] = np.array([r["mom"] for r in rows], np.float64).reshape(n, 6)
+    book = vres[n].as_dict()
+    book["vega_mom"] = book.pop("mom")
+    out[book_key].update(book)
+    return out
+
+
+def _caplet_book(caplets, kind):
+    """a strip of caplets as a book of one-flow options: flow (T_pay, 1), payer for a cap (a put on the bond), receiver
+    for a floor (a call), exercised at the reset step"""
+    cap = _caplets(caplets)
+    k = _kind(kind)
+    sw = np.zeros(len(cap), SWAPTION_DTYPE)
+    sw["T_exercise"], sw["K"], sw["N"] = cap["T_reset"], cap["K"], cap["N"]
+    sw["kind"] = {_ffi.KIND_CAP: _ffi.KIND_PAYER, _ffi.KIND_FLOOR: _ffi.KIND_RECEIVER}.get(k, -1)
+    sw["n_steps_exercise"] = cap["n_steps_reset"]
+    sw["first_flow"] = np.arange(len(cap))
+    sw["n_flows"] = 1
+    fl = np.zeros(len(cap), CASH_FLOW_DTYPE)
+    fl["T"], fl["c"] = cap["T_pay"], 1.0
+    return sw, fl
 
 
 class Rng:
@@ -443,6 +471,45 @@ class Engine:
         self._check(self._lib.hw1f_swaptions_finish(self._h, C.c_void_p(d_moments_ptr), int(n_paths_total), _ptr(sw),
                                                     len(sw), _ptr(fl), len(fl), _ptr(P_mkt), res))
         return _book_results(res, len(sw))
+
+    # -- vega of a swaption book / cap strip: sigma -/+ eps on common random numbers (no reference call site) --
+    def swaptions_vega(self, rng, swaptions, flows, P_mkt, f_mkt, eps=1e-3):
+        """What swaptions() returns (bit-identical), plus per-option arrays price_minus, se_minus, price_plus, se_plus
+        (raw prices of the models with sigma -/+ eps, which keep the curve), vega, vega_se and vega_mom[n, 6]; the
+        book's values under "book", and sim_ms."""
+        sw, fl = _swaption_book(swaptions, flows)
+        P_mkt, f_mkt = _f32(P_mkt, self.n_mat), _f32(f_mkt, self.n_mat)
+        res, vres, ms = (CapResult * (len(sw) + 1))(), (BookVega * (len(sw) + 1))(), C.c_float()
+        self._check(self._lib.hw1f_swaptions_vega(self._h, rng._h, _ptr(sw), len(sw), _ptr(fl), len(fl), _ptr(P_mkt),
+                                                  _ptr(f_mkt), float(eps), res, vres, C.byref(ms)))
+        out = _add_vega(_book_results(res, len(sw)), vres, len(sw), "book")
+        out["sim_ms"] = ms.value
+        return out
+
+    def swaptions_vega_moments(self, rng, swaptions, flows, P_mkt, f_mkt, d_moments_ptr, eps=1e-3):
+        """async: device pointer to 11 * (len(swaptions) + 1) doubles (the swaptions_moments vector first)"""
+        sw, fl = _swaption_book(swaptions, flows)
+        P_mkt, f_mkt = _f32(P_mkt, self.n_mat), _f32(f_mkt, self.n_mat)
+        self._check(self._lib.hw1f_swaptions_vega_moments(self._h, rng._h, _ptr(sw), len(sw), _ptr(fl), len(fl),
+                                                          _ptr(P_mkt), _ptr(f_mkt), float(eps),
+                                                          C.c_void_p(d_moments_ptr)))
+
+    def swaptions_vega_finish(self, d_moments_ptr, n_paths_total, swaptions, flows, P_mkt, eps=1e-3):
+        sw, fl = _swaption_book(swaptions, flows)
+        P_mkt = _f32(P_mkt, self.n_mat)
+        res, vres = (CapResult * (len(sw) + 1))(), (BookVega * (len(sw) + 1))()
+        self._check(self._lib.hw1f_swaptions_vega_finish(self._h, C.c_void_p(d_moments_ptr), int(n_paths_total),
+                                                         _ptr(sw), len(sw), _ptr(fl), len(fl), _ptr(P_mkt), float(eps),
+                                                         res, vres))
+        return _add_vega(_book_results(res, len(sw)), vres, len(sw), "book")
+
+    def cap_floor_vega(self, rng, caplets, P_mkt, f_mkt, kind="cap", eps=1e-3):
+        """What cap_floor() returns (the strip under "strip"), plus the vega arrays of swaptions_vega(): the strip is
+        priced as the book of its one-flow options (a one-flow option performs the caplet's float operations)."""
+        sw, fl = _caplet_book(caplets, kind)
+        out = self.swaptions_vega(rng, sw, fl, P_mkt, f_mkt, eps=eps)
+        out["strip"] = out.pop("book")
+        return out
 
     # -- Q3 (src/3_sensitivity_analysis.cu) --
     def vega_pathwise(self, rng, P_mkt, f_mkt, S1=5.0, S2=10.0, K=None, n_steps_S1=-1):

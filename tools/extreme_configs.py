@@ -6,6 +6,7 @@ import hw1f_b200 as hw
 from oracle_lib import Oracle
 import cap_oracle
 import swaption_oracle
+import swaption_vega_oracle
 
 
 def cap_strip(eng):
@@ -45,6 +46,18 @@ def swaption_vs_oracle(eng, over, n, c):
     return {"book_price_cv": got["book"]["price_cv"], "worst_rel_vs_oracle": float(np.abs(mom / ref - 1).max())}
 
 
+def swaption_vega_vs_oracle(eng, over, n, c):
+    sw, fl = swaption_book(eng)
+    got = eng.swaptions_vega(hw.Rng(8, n), sw, fl, c["P"], c["f"], eps=1e-3)
+    ref, _ = swaption_vega_oracle.vega_moments(Oracle(**over), 8, n, sw, fl, c["P"], c["f"], 1e-3)
+    base = np.vstack([got["mom"], np.asarray(got["book"]["mom"])[None, :]])
+    vega = np.vstack([got["vega_mom"], np.asarray(got["book"]["vega_mom"])[None, :]])
+    rb, rv = swaption_vega_oracle.split(ref, len(sw))
+    return {"book_vega": got["book"]["vega"], "book_vega_se": got["book"]["vega_se"],
+            "worst_rel_vs_oracle": float(max(np.abs(base / rb - 1).max(), np.abs(vega[:, :4] / rv[:, :4] - 1).max())),
+            "worst_D_gap_over_se": float(np.max(np.abs(vega[:, 4] - rv[:, 4]) / np.sqrt(rv[:, 5])))}
+
+
 for over in (dict(n_steps=8184, n_mat=1024), dict(n_steps=1023, n_mat=1024, T_final=10.23), dict(n_steps=2, n_mat=3, T_final=0.5), dict(n_steps=8192, n_mat=513)):
   for mode in (0, 1):
     eng = hw.Engine(device=0, params=hw.default_params(**over)); eng.set_mode(mode)
@@ -61,6 +74,7 @@ for over in (dict(n_steps=8184, n_mat=1024), dict(n_steps=1023, n_mat=1024, T_fi
                      ("batch", lambda: eng.zbc_cv_batch([1, 2], n, c["P"], c["f"], S1=S1, S2=S2, n_steps_S1=ns)[0][0]),
                      ("cap_floor", lambda: cap_vs_oracle(eng, over, n, c)),
                      ("swaptions", lambda: swaption_vs_oracle(eng, over, n, c)),
+                     ("swaptions_vega", lambda: swaption_vega_vs_oracle(eng, over, n, c)),
                      ("paths", lambda: eng.sample_paths(hw.Rng(5, n), 4).shape)):
         try:
             print("   ", name, fn())
