@@ -81,7 +81,24 @@ int hw1f_engine_device(const hw1f_engine* eng, int* device);
  *   HW1F_MODE_DECOMPOSED (default): the model is linear in the shocks, so the +G/-G twins, the
  *       sigma-bumped twins and the pathwise tangent are all (noise-free part) +/- scale * h with ONE
  *       shared noise recursion h' = h e^{-a dt} + G per stream; per-path values differ from the
- *       reference by float rounding only (~1e-7 relative; north-star tolerance 1e-5). */
+ *       reference by float rounding only.
+ *   Accuracy, measured pair by pair against a double-precision evaluation of the scheme on a B200
+ *   (tests/test_gpu_f64.py, both modes): every summand x (a discount factor, payoff, control or tangent term) is within
+ *   rel (|x| + y) of the exact value, y = D Bnd for an option payoff (its kink), with the per-pair relative bound of
+ *   tests/f64_reference.py
+ *       rel = 5 (2^-24 sqrt(n) |I| + 2e-6 sd(I)) + 5 (2^-24 |r| + 2e-6 sd(r)) B + 5 2^-24 sqrt(n_flows) + 7.2e-7,
+ *   n the steps to the evaluation, sd(.) the model's noise standard deviations: 1.1e-5 at most on the default model,
+ *   more for paths with a large |I| (4.7e-5 at a = 0.001, sigma = 0.1).  Reference order used at most 0.86 of it,
+ *   decomposed mode 0.51 inside its domain.
+ *   Decomposed mode rebuilds the noise part of I as (dt/2) sig_st (qA W - qB h) with qA = 2/(1-e^{-a dt}) and W a sum
+ *   of n normals: its rounding error grows like w n with w = dt sig_st / (1 - e^{-a dt}).  The simulating calls return
+ *   HW1F_ERR_UNSUPPORTED in this mode for n_steps w > 250 (measured inside the bound at 200 on 1000 steps and at 233 on
+ *   8184 steps; outside at 1000: a = 0.01, sigma = 0.1 on the default grid, 1.8x the bound and a 2.5e-5 bias of the mean
+ *   discount factor).  Reference order takes every model.
+ *   Both modes: the drift tables restate the reference's float expressions (compute_drift_tables), which cancel as
+ *   a dt -> 0.  Against the exact integrals they move the noise-free I(10) by 3e-8 at a = 1, 5e-6 at a = 0.1,
+ *   1.2e-5 at a = 0.05, 1e-3 at a = 0.01 and 9e-2 at a = 0.001 (dt = 0.01; tests/test_f64_reference.py).  They are kept
+ *   for parity with the reference (INTEGRATION.md, section 4). */
 #define HW1F_MODE_REFERENCE_ORDER 0
 #define HW1F_MODE_DECOMPOSED 1
 int hw1f_engine_set_mode(hw1f_engine* eng, int mode);

@@ -509,6 +509,30 @@ int require_model(hw1f_engine* e)
     return HW1F_OK;
 }
 
+// Decomposed mode rebuilds the noise part of I as c q with q = qA W - qB h, qA = 2/(1-e), qB = qA - 1 (hw1f_kernels_fast.cuh):
+// one float rounding of W moves I by about c qA ulp(W), with c qA = w = dt sig_st / (1 - e).  W is a sum of n normals, so
+// ulp(W) grows like sqrt(n) and the rounding error W accumulates over n steps like u n: the error of I grows like w n.
+// Compared pair by pair with a double-precision evaluation of the scheme (tests/test_gpu_f64.py), the kernels stay inside
+// the per-pair float bound at w n = 200 (a = 0.05, sigma = 0.1 on 1000 steps) and at w n = 233 (a = 0.05,
+// sigma = 0.045 on 8184 steps), and leave it at w n = 1000 (a = 0.01, sigma = 0.1 on 1000 steps: 1.8 x the bound, and a
+// bias of 2.5e-5 of the mean discount factor over 2^18 pairs).  Simulating calls refuse models with w n_steps > 250 in
+// decomposed mode; reference order takes every model.
+constexpr double kDecompMaxNoiseWeightSteps = 250.0;
+
+int require_model_sim(hw1f_engine* e)
+{
+    HW_TRY(require_model(e));
+    if (e->mode == HW1F_MODE_DECOMPOSED) {
+        const double w = (double)e->dt * (double)e->sig_st / (1.0 - (double)e->exp_adt) * (double)e->p.n_steps;
+        if (!(w <= kDecompMaxNoiseWeightSteps)) {
+            e->err = "decomposed mode is accurate only for n_steps dt sig_st / (1 - exp(-a dt)) <= 250 (this model: " +
+                     std::to_string(w) + "); use HW1F_MODE_REFERENCE_ORDER";
+            return HW1F_ERR_UNSUPPORTED;
+        }
+    }
+    return HW1F_OK;
+}
+
 int resolve_steps(hw1f_engine* e, float S1, int32_t n_in, int32_t* n_out)
 {
     if (n_in >= 0) { *n_out = n_in; }
@@ -1408,7 +1432,7 @@ static int read_curve(hw1f_engine* e, int area, int scen, float* P, float* f, fl
 
 int hw1f_bond_curve_moments(hw1f_engine* e, hw1f_rng* rng, double* d_moments)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !d_moments) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     Finish fin;
@@ -1434,7 +1458,7 @@ int hw1f_bond_curve_finish(hw1f_engine* e, const double* d_moments, uint64_t n_p
 
 int hw1f_bond_curve(hw1f_engine* e, hw1f_rng* rng, float* P, float* f, float* P_se, float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !P || !f) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     HW_CUDA(e, e->d_moments.ensure(4 * (size_t)e->p.n_mat * kMaxRuns));
@@ -1478,7 +1502,7 @@ static int lane_of(hw1f_engine* e, int32_t slot, hw1f_engine** lane)
 
 int hw1f_bond_curve_submit(hw1f_engine* e, hw1f_rng* rng, int32_t slot)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng) return HW1F_ERR_INVALID;
     HW_REQUIRE(e, slot >= 0 && slot < kAsyncSlots, "slot outside [0, HW1F_ASYNC_SLOTS)");
     HW_REQUIRE(e, !e->slot_busy[slot], "result slot still in flight: collect it first");
@@ -1631,7 +1655,7 @@ static int zbc_run(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, c
 int hw1f_zbc_cv_moments(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const float* P_mkt,
                         const float* f_mkt, int32_t n_steps_S1, double* d_moments)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     int32_t n = 0;
@@ -1658,7 +1682,7 @@ int hw1f_zbc_cv_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths
 int hw1f_zbc_cv(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const float* P_mkt, const float* f_mkt,
                 int32_t n_steps_S1, hw1f_zbc_result* out, float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !out || !P_mkt || !f_mkt) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     int32_t n = 0;
@@ -1683,7 +1707,7 @@ int hw1f_zbc_cv_batch(hw1f_engine* e, const uint64_t* seeds, int32_t n_runs, uin
                       float K, const float* P_mkt, const float* f_mkt, int32_t n_steps_S1, hw1f_zbc_result* out,
                       float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!seeds || !out || !P_mkt || !f_mkt) return HW1F_ERR_INVALID;
     HW_REQUIRE(e, 2 * n_paths < (1ull << 31), "the reference's int N_total needs 2*n_paths < 2^31");
     HW_CUDA(e, cudaSetDevice(e->device));
@@ -1730,7 +1754,7 @@ static int pathwise_run(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float
 int hw1f_vega_pathwise_moments(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const float* P_mkt,
                                const float* f_mkt, int32_t n_steps_S1, double* d_moments)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     int32_t n = 0;
@@ -1752,7 +1776,7 @@ static void pathwise_result(const double mom[2], uint64_t n_paths, hw1f_vega_res
 int hw1f_vega_pathwise(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const float* P_mkt,
                        const float* f_mkt, int32_t n_steps_S1, hw1f_vega_result* out)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !out || !P_mkt || !f_mkt) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     int32_t n = 0;
@@ -1778,7 +1802,7 @@ int hw1f_vega_pathwise_batch(hw1f_engine* e, const uint64_t* seeds, int32_t n_ru
                              float S2, float K, const float* P_mkt, const float* f_mkt, int32_t n_steps_S1,
                              float* vega, float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!seeds || !vega || !P_mkt || !f_mkt) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     int32_t n = 0;
@@ -1878,7 +1902,7 @@ static void recal_result(hw1f_engine* e, int res_area, uint64_t n_paths, float e
 int hw1f_vega_fd(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const float* P_mkt, const float* f_mkt,
                  float eps, int32_t n_steps_S1, hw1f_vega_result* out)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !out || !P_mkt || !f_mkt) return HW1F_ERR_INVALID;
     HW_REQUIRE(e, 2 * rng->n_paths < (1ull << 31), "the reference's int N_total needs 2*n_paths < 2^31");
     HW_CUDA(e, cudaSetDevice(e->device));
@@ -1907,7 +1931,7 @@ int hw1f_vega_fd(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, con
 int hw1f_vega_fd_recalibrated(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, float eps,
                               int32_t n_steps_S1, hw1f_vega_result* out)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !out) return HW1F_ERR_INVALID;
     HW_REQUIRE(e, 2 * rng->n_paths < (1ull << 31), "the reference's int N_total needs 2*n_paths < 2^31");
     HW_CUDA(e, cudaSetDevice(e->device));
@@ -1935,7 +1959,7 @@ int hw1f_vega_fd_recalibrated(hw1f_engine* e, hw1f_rng* rng, float S1, float S2,
 int hw1f_vega(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const float* P_mkt, const float* f_mkt,
               float eps, int32_t n_steps_S1, hw1f_vega_result* out)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !out || !P_mkt || !f_mkt) return HW1F_ERR_INVALID;
     HW_REQUIRE(e, 2 * rng->n_paths < (1ull << 31), "the reference's int N_total needs 2*n_paths < 2^31");
     HW_CUDA(e, cudaSetDevice(e->device));
@@ -2064,7 +2088,7 @@ int hw1f_vega(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const 
 static int fused_launch(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const float* P_mkt,
                         const float* f_mkt, bool fd, float eps, int32_t n_steps_S1, double* d_moments, const Finish& fin)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
     HW_CUDA(e, cudaSetDevice(e->device));
     int32_t n = 0;
@@ -2194,7 +2218,7 @@ int hw1f_fused(hw1f_engine* e, hw1f_rng* rng, float S1, float S2, float K, const
                float eps, int32_t n_steps_S1, float* P, float* f, float* P_se, hw1f_zbc_result* zbc,
                hw1f_vega_result* vega, float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !P_mkt || !f_mkt || !P || !f || !zbc || !vega) return HW1F_ERR_INVALID;
     HW_REQUIRE(e, eps > 0.0f, "hw1f_fused needs eps > 0 (the FD bumps ride on the same launch)");
     HW_CUDA(e, cudaSetDevice(e->device));
@@ -2344,7 +2368,7 @@ static void cap_results(const hw1f_engine* e, const double* mom, uint64_t n_pair
 int hw1f_cap_floor_moments(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n,
                            const float* P_mkt, const float* f_mkt, double* d_moments)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !caps || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
     std::vector<int> steps;
     HW_TRY(cap_validate(e, kind, caps, n, steps));
@@ -2373,7 +2397,7 @@ int hw1f_cap_floor_finish(hw1f_engine* e, const double* d_moments, uint64_t n_pa
 int hw1f_cap_floor(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n, const float* P_mkt,
                    const float* f_mkt, hw1f_cap_result* out, float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !caps || !P_mkt || !f_mkt || !out) return HW1F_ERR_INVALID;
     std::vector<int> steps;
     HW_TRY(cap_validate(e, kind, caps, n, steps));
@@ -2513,7 +2537,7 @@ int hw1f_swaptions_moments(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* s
                            const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
                            double* d_moments)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !sw || !flows || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
     std::vector<int> steps;
     int rows = 0;
@@ -2545,7 +2569,7 @@ int hw1f_swaptions_finish(hw1f_engine* e, const double* d_moments, uint64_t n_pa
 int hw1f_swaptions(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
                    int32_t n_flows, const float* P_mkt, const float* f_mkt, hw1f_cap_result* out, float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !sw || !flows || !P_mkt || !f_mkt || !out) return HW1F_ERR_INVALID;
     std::vector<int> steps;
     int rows = 0;
@@ -2736,7 +2760,7 @@ int hw1f_swaptions_vega_moments(hw1f_engine* e, hw1f_rng* rng, const hw1f_swapti
                                 const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
                                 float eps, double* d_moments)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !sw || !flows || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
     std::vector<int> steps;
     int rows = 0;
@@ -2772,7 +2796,7 @@ int hw1f_swaptions_vega(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, 
                         int32_t n_flows, const float* P_mkt, const float* f_mkt, float eps, hw1f_cap_result* out,
                         hw1f_book_vega* vega, float* sim_ms)
 {
-    HW_TRY(require_model(e));
+    HW_TRY(require_model_sim(e));
     if (!rng || !sw || !flows || !P_mkt || !f_mkt || !out || !vega) return HW1F_ERR_INVALID;
     std::vector<int> steps;
     int rows = 0;
