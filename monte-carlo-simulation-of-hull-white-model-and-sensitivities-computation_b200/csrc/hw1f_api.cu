@@ -19,7 +19,6 @@
 #include "hw1f_kernels.cuh"
 #include "hw1f_kernels_extra.cuh"
 #include "hw1f_kernels_fast.cuh"
-#include "hw1f_kernels_cap.cuh"
 #include "hw1f_kernels_swaption.cuh"
 #include "hw1f_kernels_book_vega.cuh"
 #include "hw1f_tail.cuh"
@@ -1005,8 +1004,6 @@ int init_kernels(hw1f_engine* e)
     HW_CUDA(e, opt_in(zbc_sum_kernel<1>, b));
     HW_CUDA(e, opt_in(zbc_sum_kernel<2>, b));
     HW_CUDA(e, opt_in(zbc_sum_kernel<3>, b));
-    HW_CUDA(e, opt_in(cap_kernel<0>, b));
-    HW_CUDA(e, opt_in(cap_kernel<1>, b));
     HW_CUDA(e, opt_in(swaption_kernel<0>, b));
     HW_CUDA(e, opt_in(swaption_kernel<1>, b));
     HW_CUDA(e, opt_in(book_vega_kernel<0>, b));
@@ -2274,47 +2271,6 @@ static int cap_validate(hw1f_engine* e, int32_t kind, const hw1f_caplet* caps, i
     return HW1F_OK;
 }
 
-// one staged upload of [caplet table | P_mkt | f_mkt], the launch and its tail
-static int cap_run(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n,
-                   const std::vector<int>& steps, const float* P_mkt, const float* f_mkt, double* d_moments,
-                   const Finish& fin)
-{
-    const int nm = e->p.n_mat, nq = 5 * (n + 1);
-    const size_t tab = ((size_t)n * sizeof(CapletDev) + 255) & ~(size_t)255;
-    std::vector<char> h(tab + 2 * (size_t)nm * sizeof(float), 0);
-    CapletDev* cd = reinterpret_cast<CapletDev*>(h.data());
-    for (int i = 0; i < n; ++i) {
-        cd[i].T_reset = caps[i].T_reset;
-        cd[i].T_pay = caps[i].T_pay;
-        cd[i].K = caps[i].K;
-        cd[i].N = caps[i].N;
-        cd[i].m = (float)e->det_m[0][steps[i]];
-        cd[i].Im = (float)e->det_I[0][steps[i]];
-        cd[i].step = steps[i];
-        cd[i].pad = 0;
-    }
-    memcpy(h.data() + tab, P_mkt, nm * sizeof(float));
-    memcpy(h.data() + tab + nm * sizeof(float), f_mkt, nm * sizeof(float));
-    const int decomp = e->mode == HW1F_MODE_DECOMPOSED;
-    const size_t smem = cap_smem_bytes(decomp, n, steps[n - 1]);
-    HW_TRY(decomp ? set_smem(e, cap_kernel<1>, smem) : set_smem(e, cap_kernel<0>, smem));
-    HW_CUDA(e, e->d_cap.ensure(h.size()));
-    HW_TRY(upload(e, e->d_cap.p, h.data(), h.size()));
-    Launch L;
-    HW_TRY(prepare_launch(e, &rng->seed, 1, rng->first_path, rng->n_paths, rng->offset, &L));
-    HW_CUDA(e, e->d_partials.ensure((size_t)L.grid_x * nq));
-    const ScenDev sc = scen_dev(e, e->p.sigma, e->sig_st, 0);
-    const CapletDev* d_caps = reinterpret_cast<const CapletDev*>(e->d_cap.p);
-    const float* d_P = reinterpret_cast<const float*>(e->d_cap.p + tab);
-    const float sgn = (kind == HW1F_KIND_CAP) ? -1.0f : 1.0f;
-    HW_CUDA(e, launch_k(decomp ? cap_kernel<1> : cap_kernel<0>, dim3(L.grid_x, 1), kThreads, smem, e->stream, true, L.g,
-                        L.seeds, model_dev(e), sc, d_caps, (int)n, d_P, d_P + nm, sgn, L.lead, e->d_partials.p));
-    HW_TRY(check_launch(e, "cap_kernel"));
-    HW_TRY(launch_tail(e, L, L.g.n_paths, nq, 0, nullptr, nullptr, 0.f, d_moments, nq, nq, fin));
-    rng->offset += (uint64_t)steps[n - 1];
-    return HW1F_OK;
-}
-
 // P_mkt(T) as interp_mkt evaluates it on the device (IEEE single operations, one fused multiply-add each)
 static float host_interp_mkt(const hw1f_engine* e, const float* data, float T)
 {
@@ -2351,71 +2307,6 @@ static void cap_algebra(const double mom[5], uint64_t n_pairs, double control_me
     r->se_cv = sqrt(vcv / n);
     r->corr = (vxx > 0.0 && vyy > 0.0) ? cxy / sqrt(vxx * vyy) : 0.0;
     r->control_mean = control_mean;
-}
-
-static void cap_results(const hw1f_engine* e, const double* mom, uint64_t n_pairs, const hw1f_caplet* caps, int32_t n,
-                        const float* P_mkt, hw1f_cap_result* out)
-{
-    double strip_mean = 0.0;
-    for (int i = 0; i < n; ++i) {
-        const double cm = (double)caps[i].N * (double)host_interp_mkt(e, P_mkt, caps[i].T_pay);
-        strip_mean += cm;
-        cap_algebra(mom + 5 * i, n_pairs, cm, out + i);
-    }
-    cap_algebra(mom + 5 * n, n_pairs, strip_mean, out + n);
-}
-
-int hw1f_cap_floor_moments(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n,
-                           const float* P_mkt, const float* f_mkt, double* d_moments)
-{
-    HW_TRY(require_model_sim(e));
-    if (!rng || !caps || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
-    std::vector<int> steps;
-    HW_TRY(cap_validate(e, kind, caps, n, steps));
-    HW_CUDA(e, cudaSetDevice(e->device));
-    Finish fin;
-    fin.exchange = true;   // with peers attached (hw1f_comm_attach) the last block all-reduces the vector itself
-    return cap_run(e, rng, kind, caps, n, steps, P_mkt, f_mkt, d_moments, fin);
-}
-
-int hw1f_cap_floor_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths_total, const hw1f_caplet* caps,
-                          int32_t n, const float* P_mkt, hw1f_cap_result* out)
-{
-    HW_TRY(require_model(e));
-    if (!d_moments || !caps || !P_mkt || !out) return HW1F_ERR_INVALID;
-    HW_REQUIRE(e, n_paths_total >= 1 && n_paths_total < (1ull << 40), "n_paths_total outside [1, 2^40)");
-    std::vector<int> steps;
-    HW_TRY(cap_validate(e, HW1F_KIND_CAP, caps, n, steps));
-    HW_CUDA(e, cudaSetDevice(e->device));
-    std::vector<double> mom(5 * (size_t)(n + 1));
-    HW_TRY(download(e, mom.data(), d_moments, mom.size() * sizeof(double)));
-    HW_TRY(require_finite(e, mom.data(), (int)mom.size()));
-    cap_results(e, mom.data(), n_paths_total, caps, n, P_mkt, out);
-    return HW1F_OK;
-}
-
-int hw1f_cap_floor(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n, const float* P_mkt,
-                   const float* f_mkt, hw1f_cap_result* out, float* sim_ms)
-{
-    HW_TRY(require_model_sim(e));
-    if (!rng || !caps || !P_mkt || !f_mkt || !out) return HW1F_ERR_INVALID;
-    std::vector<int> steps;
-    HW_TRY(cap_validate(e, kind, caps, n, steps));
-    HW_CUDA(e, cudaSetDevice(e->device));
-    const size_t nq = 5 * (size_t)(n + 1);
-    HW_CUDA(e, e->d_moments.ensure(std::max(4 * (size_t)e->p.n_mat * kMaxRuns, nq)));
-    HW_TRY(warm_geometry(e, rng));
-    Finish fin;
-    fin.host_mom = res_mom(e, 0);   // the result area holds at least 512 doubles
-    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev0, e->stream));
-    HW_TRY(cap_run(e, rng, kind, caps, n, steps, P_mkt, f_mkt, e->d_moments.p, fin));
-    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev1, e->stream));
-    HW_TRY(wait_results(e));
-    std::vector<double> mom(res_mom(e, 0), res_mom(e, 0) + nq);
-    HW_TRY(require_finite(e, mom.data(), (int)nq));
-    cap_results(e, mom.data(), rng->n_paths, caps, n, P_mkt, out);
-    if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
-    return HW1F_OK;
 }
 
 // ---- European swaptions -------------------------------------------------------------------------
@@ -2466,18 +2357,11 @@ static int swaption_validate(hw1f_engine* e, const hw1f_swaption* sw, int32_t n,
     return HW1F_OK;
 }
 
-// one staged upload of [option table | flow table | P_mkt | f_mkt], the launch and its tail.  The flow table holds each
-// option's flows in its own contiguous rows, with its exercise date beside them.
-static int swaption_run(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
-                        const std::vector<int>& steps, int n_rows, const float* P_mkt, const float* f_mkt,
-                        double* d_moments, const Finish& fin)
+// the option and flow tables of a book as the kernels read them: each option's flows in its own contiguous rows, with
+// its exercise date beside them
+static void fill_book_tables(const hw1f_engine* e, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                             const std::vector<int>& steps, SwaptionDev* sd, SwFlowDev* fd)
 {
-    const int nm = e->p.n_mat, nq = 5 * (n + 1);
-    const size_t tab = ((size_t)n * sizeof(SwaptionDev) + 255) & ~(size_t)255;
-    const size_t ftab = ((size_t)n_rows * sizeof(SwFlowDev) + 255) & ~(size_t)255;
-    std::vector<char> h(tab + ftab + 2 * (size_t)nm * sizeof(float), 0);
-    SwaptionDev* sd = reinterpret_cast<SwaptionDev*>(h.data());
-    SwFlowDev* fd = reinterpret_cast<SwFlowDev*>(h.data() + tab);
     int row = 0;
     for (int i = 0; i < n; ++i) {
         sd[i].T_e = sw[i].T_exercise;
@@ -2495,6 +2379,19 @@ static int swaption_run(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, 
             fd[row].c = flows[sw[i].first_flow + j].c;
         }
     }
+}
+
+// one staged upload of [option table | flow table | P_mkt | f_mkt], the launch and its tail
+static int swaption_run(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                        const std::vector<int>& steps, int n_rows, const float* P_mkt, const float* f_mkt,
+                        double* d_moments, const Finish& fin)
+{
+    const int nm = e->p.n_mat, nq = 5 * (n + 1);
+    const size_t tab = ((size_t)n * sizeof(SwaptionDev) + 255) & ~(size_t)255;
+    const size_t ftab = ((size_t)n_rows * sizeof(SwFlowDev) + 255) & ~(size_t)255;
+    std::vector<char> h(tab + ftab + 2 * (size_t)nm * sizeof(float), 0);
+    fill_book_tables(e, sw, n, flows, steps, reinterpret_cast<SwaptionDev*>(h.data()),
+                     reinterpret_cast<SwFlowDev*>(h.data() + tab));
     memcpy(h.data() + tab + ftab, P_mkt, nm * sizeof(float));
     memcpy(h.data() + tab + ftab + nm * sizeof(float), f_mkt, nm * sizeof(float));
     const int decomp = e->mode == HW1F_MODE_DECOMPOSED;
@@ -2533,6 +2430,49 @@ static void swaption_results(const hw1f_engine* e, const double* mom, uint64_t n
     cap_algebra(mom + 5 * n, n_pairs, book_mean, out + n);
 }
 
+// the bodies of the entry points below, on a book that has passed its checks: the swaptions' own, or a cap strip's
+static int book_moments(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                        const std::vector<int>& steps, int n_rows, const float* P_mkt, const float* f_mkt,
+                        double* d_moments)
+{
+    HW_CUDA(e, cudaSetDevice(e->device));
+    Finish fin;
+    fin.exchange = true;   // with peers attached (hw1f_comm_attach) the last block all-reduces the vector itself
+    return swaption_run(e, rng, sw, n, flows, steps, n_rows, P_mkt, f_mkt, d_moments, fin);
+}
+
+static int book_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths_total, const hw1f_swaption* sw,
+                       int32_t n, const hw1f_cash_flow* flows, const float* P_mkt, hw1f_cap_result* out)
+{
+    HW_CUDA(e, cudaSetDevice(e->device));
+    std::vector<double> mom(5 * (size_t)(n + 1));
+    HW_TRY(download(e, mom.data(), d_moments, mom.size() * sizeof(double)));
+    HW_TRY(require_finite(e, mom.data(), (int)mom.size()));
+    swaption_results(e, mom.data(), n_paths_total, sw, n, flows, P_mkt, out);
+    return HW1F_OK;
+}
+
+static int book_price(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
+                      const std::vector<int>& steps, int n_rows, const float* P_mkt, const float* f_mkt,
+                      hw1f_cap_result* out, float* sim_ms)
+{
+    HW_CUDA(e, cudaSetDevice(e->device));
+    const size_t nq = 5 * (size_t)(n + 1);
+    HW_CUDA(e, e->d_moments.ensure(std::max(4 * (size_t)e->p.n_mat * kMaxRuns, nq)));
+    HW_TRY(warm_geometry(e, rng));
+    Finish fin;
+    fin.host_mom = res_mom(e, 0);   // the result area holds at least 512 doubles
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev0, e->stream));
+    HW_TRY(swaption_run(e, rng, sw, n, flows, steps, n_rows, P_mkt, f_mkt, e->d_moments.p, fin));
+    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev1, e->stream));
+    HW_TRY(wait_results(e));
+    std::vector<double> mom(res_mom(e, 0), res_mom(e, 0) + nq);
+    HW_TRY(require_finite(e, mom.data(), (int)nq));
+    swaption_results(e, mom.data(), rng->n_paths, sw, n, flows, P_mkt, out);
+    if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
+    return HW1F_OK;
+}
+
 int hw1f_swaptions_moments(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n,
                            const hw1f_cash_flow* flows, int32_t n_flows, const float* P_mkt, const float* f_mkt,
                            double* d_moments)
@@ -2542,10 +2482,7 @@ int hw1f_swaptions_moments(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* s
     std::vector<int> steps;
     int rows = 0;
     HW_TRY(swaption_validate(e, sw, n, flows, n_flows, steps, &rows));
-    HW_CUDA(e, cudaSetDevice(e->device));
-    Finish fin;
-    fin.exchange = true;   // with peers attached (hw1f_comm_attach) the last block all-reduces the vector itself
-    return swaption_run(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, d_moments, fin);
+    return book_moments(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, d_moments);
 }
 
 int hw1f_swaptions_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths_total, const hw1f_swaption* sw,
@@ -2558,12 +2495,7 @@ int hw1f_swaptions_finish(hw1f_engine* e, const double* d_moments, uint64_t n_pa
     std::vector<int> steps;
     int rows = 0;
     HW_TRY(swaption_validate(e, sw, n, flows, n_flows, steps, &rows));
-    HW_CUDA(e, cudaSetDevice(e->device));
-    std::vector<double> mom(5 * (size_t)(n + 1));
-    HW_TRY(download(e, mom.data(), d_moments, mom.size() * sizeof(double)));
-    HW_TRY(require_finite(e, mom.data(), (int)mom.size()));
-    swaption_results(e, mom.data(), n_paths_total, sw, n, flows, P_mkt, out);
-    return HW1F_OK;
+    return book_finish(e, d_moments, n_paths_total, sw, n, flows, P_mkt, out);
 }
 
 int hw1f_swaptions(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32_t n, const hw1f_cash_flow* flows,
@@ -2574,21 +2506,70 @@ int hw1f_swaptions(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw, int32
     std::vector<int> steps;
     int rows = 0;
     HW_TRY(swaption_validate(e, sw, n, flows, n_flows, steps, &rows));
-    HW_CUDA(e, cudaSetDevice(e->device));
-    const size_t nq = 5 * (size_t)(n + 1);
-    HW_CUDA(e, e->d_moments.ensure(std::max(4 * (size_t)e->p.n_mat * kMaxRuns, nq)));
-    HW_TRY(warm_geometry(e, rng));
-    Finish fin;
-    fin.host_mom = res_mom(e, 0);   // the result area holds at least 512 doubles
-    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev0, e->stream));
-    HW_TRY(swaption_run(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, e->d_moments.p, fin));
-    if (sim_ms) HW_CUDA(e, cudaEventRecord(e->ev1, e->stream));
-    HW_TRY(wait_results(e));
-    std::vector<double> mom(res_mom(e, 0), res_mom(e, 0) + nq);
-    HW_TRY(require_finite(e, mom.data(), (int)nq));
-    swaption_results(e, mom.data(), rng->n_paths, sw, n, flows, P_mkt, out);
-    if (sim_ms) HW_CUDA(e, cudaEventElapsedTime(sim_ms, e->ev0, e->ev1));
-    return HW1F_OK;
+    return book_price(e, rng, sw, n, flows, steps, rows, P_mkt, f_mkt, out, sim_ms);
+}
+
+// ---- caps and floors as books of one-flow options -----------------------------------------------
+static_assert(HW1F_MAX_CAPLETS <= HW1F_MAX_SWAPTIONS, "a strip must fit a book");
+
+// option i exercises at T_reset into flow i = (T_pay, c = 1): a put on the bond (payer) for a cap, a call (receiver)
+// for a floor.  With c = 1 the book performs a caplet's float operations, and its control mean is N P_mkt(T_pay).
+static void caplet_book(int32_t kind, const hw1f_caplet* caps, int32_t n, const std::vector<int>& steps,
+                        std::vector<hw1f_swaption>& sw, std::vector<hw1f_cash_flow>& flows)
+{
+    sw.assign(n, hw1f_swaption{});
+    flows.assign(n, hw1f_cash_flow{});
+    for (int i = 0; i < n; ++i) {
+        sw[i].T_exercise = caps[i].T_reset;
+        sw[i].K = caps[i].K;
+        sw[i].N = caps[i].N;
+        sw[i].kind = (kind == HW1F_KIND_CAP) ? HW1F_KIND_PAYER : HW1F_KIND_RECEIVER;
+        sw[i].n_steps_exercise = steps[i];
+        sw[i].first_flow = i;
+        sw[i].n_flows = 1;
+        flows[i].T = caps[i].T_pay;
+        flows[i].c = 1.0f;
+    }
+}
+
+int hw1f_cap_floor_moments(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n,
+                           const float* P_mkt, const float* f_mkt, double* d_moments)
+{
+    HW_TRY(require_model_sim(e));
+    if (!rng || !caps || !P_mkt || !f_mkt || !d_moments) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    HW_TRY(cap_validate(e, kind, caps, n, steps));
+    std::vector<hw1f_swaption> sw;
+    std::vector<hw1f_cash_flow> flows;
+    caplet_book(kind, caps, n, steps, sw, flows);
+    return book_moments(e, rng, sw.data(), n, flows.data(), steps, n, P_mkt, f_mkt, d_moments);
+}
+
+int hw1f_cap_floor_finish(hw1f_engine* e, const double* d_moments, uint64_t n_paths_total, const hw1f_caplet* caps,
+                          int32_t n, const float* P_mkt, hw1f_cap_result* out)
+{
+    HW_TRY(require_model(e));
+    if (!d_moments || !caps || !P_mkt || !out) return HW1F_ERR_INVALID;
+    HW_REQUIRE(e, n_paths_total >= 1 && n_paths_total < (1ull << 40), "n_paths_total outside [1, 2^40)");
+    std::vector<int> steps;
+    HW_TRY(cap_validate(e, HW1F_KIND_CAP, caps, n, steps));
+    std::vector<hw1f_swaption> sw;
+    std::vector<hw1f_cash_flow> flows;
+    caplet_book(HW1F_KIND_CAP, caps, n, steps, sw, flows);
+    return book_finish(e, d_moments, n_paths_total, sw.data(), n, flows.data(), P_mkt, out);
+}
+
+int hw1f_cap_floor(hw1f_engine* e, hw1f_rng* rng, int32_t kind, const hw1f_caplet* caps, int32_t n, const float* P_mkt,
+                   const float* f_mkt, hw1f_cap_result* out, float* sim_ms)
+{
+    HW_TRY(require_model_sim(e));
+    if (!rng || !caps || !P_mkt || !f_mkt || !out) return HW1F_ERR_INVALID;
+    std::vector<int> steps;
+    HW_TRY(cap_validate(e, kind, caps, n, steps));
+    std::vector<hw1f_swaption> sw;
+    std::vector<hw1f_cash_flow> flows;
+    caplet_book(kind, caps, n, steps, sw, flows);
+    return book_price(e, rng, sw.data(), n, flows.data(), steps, n, P_mkt, f_mkt, out, sim_ms);
 }
 
 // ---- vega of a swaption book: sigma -/+ eps on common random numbers in the pricing pass -----------------------
@@ -2670,27 +2651,12 @@ static int book_vega_run(hw1f_engine* e, hw1f_rng* rng, const hw1f_swaption* sw,
     SwaptionDev* sd = reinterpret_cast<SwaptionDev*>(h.data());
     BookVegaOptDev* bd = reinterpret_cast<BookVegaOptDev*>(h.data() + tab);
     SwFlowDev* fd = reinterpret_cast<SwFlowDev*>(h.data() + tab + btab);
-    int row = 0;
-    for (int i = 0; i < n; ++i) {   // the option and flow tables of swaption_run
-        sd[i].T_e = sw[i].T_exercise;
-        sd[i].K = sw[i].K;
-        sd[i].N = sw[i].N;
-        sd[i].sgn = (sw[i].kind == HW1F_KIND_PAYER) ? -1.0f : 1.0f;
-        sd[i].m = (float)e->det_m[0][steps[i]];
-        sd[i].Im = (float)e->det_I[0][steps[i]];
-        sd[i].step = steps[i];
-        sd[i].f0 = row;
-        sd[i].nf = sw[i].n_flows;
+    fill_book_tables(e, sw, n, flows, steps, sd, fd);
+    for (int i = 0; i < n; ++i)
         for (int s = 0; s < 2; ++s) {
             bd[i].m[s] = (float)e->det_m[4 + s][steps[i]];
             bd[i].Im[s] = (float)e->det_I[4 + s][steps[i]];
         }
-        for (int j = 0; j < sw[i].n_flows; ++j, ++row) {
-            fd[row].T_e = sw[i].T_exercise;
-            fd[row].T = flows[sw[i].first_flow + j].T;
-            fd[row].c = flows[sw[i].first_flow + j].c;
-        }
-    }
     char* mkt = h.data() + tab + btab + ftab;
     memcpy(mkt, P_mkt, nm * sizeof(float));
     memcpy(mkt + nm * sizeof(float), f_mkt, nm * sizeof(float));

@@ -3,11 +3,11 @@
 // estimator is the common-random-number central difference of run_finite_difference (src/3:400-446); every bumped
 // model keeps the initial curve through its own shifted drift table.
 //
-//   * Walk: that of swaption_kernel (hw1f_kernels_swaption.cuh), repeated here so that swaption_kernel's code stays
-//     exactly as it is.  DECOMP = 0 steps three twin pairs with hw_step2, one per scenario, each on its own drift table
-//     (all three staged in shared memory).  DECOMP = 1 carries the one noise recursion (h, W) all scenarios share and
-//     rebuilds, at an exercise step k, r_s(+/-) = m_s,k +/- sg_s h and I_s(+/-) = Im_s,k +/- c_s q with q computed once:
-//     a bumped scenario costs its payoffs, not another pass over the paths.
+//   * Walk: exercise_walk of swaption_kernel (hw1f_kernels_swaption.cuh), with its book prologue and moment rows.  Its
+//     step functor here steps three twin pairs with hw_step2 in reference order (DECOMP = 0), one per scenario, each on
+//     its own drift table (all three staged in shared memory).  DECOMP = 1 carries the one noise recursion (h, W) all
+//     scenarios share and rebuilds, at an exercise step k, r_s(+/-) = m_s,k +/- sg_s h and I_s(+/-) = Im_s,k +/- c_s q
+//     with q computed once: a bumped scenario costs its payoffs, not another pass over the paths.
 //   * Base scenario: the float operations of swaption_kernel -- swaption_payoffs, the same warp trees, the same Y
 //     centring and the same per-chunk double accumulation into its own partial row of 5 (n + 1) doubles -- so that its
 //     moments equal hw1f_swaptions bit for bit.
@@ -81,6 +81,16 @@ __host__ __device__ inline size_t book_vega_smem_bytes(int decomp, int n_swaptio
     return b + 64;
 }
 
+// sum X-, X-^2, X+, X+^2, D, D^2 of the warp through float warp trees into row[0, 6) of the warp's rows
+__device__ __forceinline__ void write_vega6(float* row, float2 Xm, float2 Xp, float2 D, int lane)
+{
+    const float sm = warp_sum_pair(add_(Xm.x, Xm.y), fma_(Xm.x, Xm.x, mul_(Xm.y, Xm.y)), lane);
+    const float sp = warp_sum_pair(add_(Xp.x, Xp.y), fma_(Xp.x, Xp.x, mul_(Xp.y, Xp.y)), lane);
+    const float sd = warp_sum_pair(add_(D.x, D.y), fma_(D.x, D.x, mul_(D.y, D.y)), lane);
+    row += (lane & 16) ? 1 : 0;
+    if ((lane & 15) == 0) { row[0] = sm; row[2] = sp; row[4] = sd; }
+}
+
 // partials[block][5 (n + 1)]: the base moments in the layout of swaption_kernel; partials_v[block][6 (n + 1)]: option i
 // at 6 i, the book at 6 n.  sw, flows, P_mkt, f_mkt as swaption_kernel; bo[n] the bumped noise-free tables.
 // One block per SM: 128 registers for the three scenarios' state and payoffs.
@@ -113,47 +123,20 @@ book_vega_kernel(StreamGeom g, SeedArgs seeds, ModelDev md, ScenDev sc, BookVega
             drift[n_last + i] = bv.drift[0][i];
             drift[2 * n_last + i] = bv.drift[1][i];
         }
+    for (int i = tid; i < n; i += kThreads) bs[i] = bo[i];   // bs and fa: published by book_prologue's barrier
     const MktPts none{};
-    for (int j = tid; j < n_rows; j += kThreads) {
-        // the bond plans of P(T_e, T_j) in the three scenarios: B (so negB) does not depend on sigma
-        const SwFlowDev f = flows[j];
-        const BondPlan pl = compute_plan(md, sc.sigma, sc.sig_st, f.T_e, f.T, P_mkt, f_mkt, none, 0);
+    book_prologue(md, sc, sw, n, flows, n_rows, P_mkt, f_mkt, fs, ss, [&](int j, const SwFlowDev& f) {
+        // the bumped bond plans of P(T_e, T_j): B (so negB) does not depend on sigma
         const BondPlan pm = compute_plan(md, bv.sigma[0], bv.sig_st[0], f.T_e, f.T, P_mkt, f_mkt, none, 0);
         const BondPlan pp = compute_plan(md, bv.sigma[1], bv.sig_st[1], f.T_e, f.T, P_mkt, f_mkt, none, 0);
-        SwFlowSh s;
-        s.A = pl.A; s.negB = pl.negB; s.c = f.c;
-        fs[j] = s;
         fa[j] = make_float2(pm.A, pp.A);
-    }
-    for (int i = tid; i < n; i += kThreads) bs[i] = bo[i];
-    __syncthreads();
-    for (int i = tid; i < n; i += kThreads) {
-        // the centring constant of the base control: Y of the noise-free pair
-        const SwaptionDev o = sw[i];
-        PairState ps;
-        ps.r1 = ps.r2 = splat(o.m);
-        ps.I1 = ps.I2 = splat(o.Im);
-        float2 x1, x2, y1, y2;
-        swaption_payoffs(ps, fs + o.f0, o.nf, o.K, o.sgn, x1, x2, y1, y2);
-        SwaptionSh s;
-        s.K = o.K; s.N = o.N; s.sgn = o.sgn; s.m = o.m; s.Im = o.Im;
-        s.cen = mul_(o.N, add_(y1.x, y2.x));
-        s.step = o.step; s.f0 = o.f0; s.nf = o.nf;
-        ss[i] = s;
-    }
+    });
 
-    const float2 e2 = splat(md.exp_adt), ee2 = splat(md.exp_2adt), hdt2 = splat(mul_(0.5f, md.dt));
-    const float2 sgP = splat(sc.sig_st), sgM = splat(-sc.sig_st);
-    const float cI = mul_(mul_(0.5f, md.dt), sc.sig_st);   // FastScen::c
-    float cIb[2];
-    float2 sgPb[2], sgMb[2];
+    const float2 e2 = splat(md.exp_adt), hdt2 = splat(mul_(0.5f, md.dt));
+    const float sg[3] = {sc.sig_st, bv.sig_st[0], bv.sig_st[1]};   // sigma, sigma - eps, sigma + eps
+    float cI[3];                                                    // FastScen::c of each
 #pragma unroll
-    for (int s = 0; s < 2; ++s) {
-        cIb[s] = mul_(mul_(0.5f, md.dt), bv.sig_st[s]);
-        sgPb[s] = splat(bv.sig_st[s]);
-        sgMb[s] = splat(-bv.sig_st[s]);
-    }
-    const bool writer = (lane & 15) == 0;
+    for (int s = 0; s < 3; ++s) cI[s] = mul_(mul_(0.5f, md.dt), sg[s]);
 
     asm volatile("griddepcontrol.wait;" ::: "memory");   // the per-launch table U of prep_lo_kernel
 
@@ -162,117 +145,38 @@ book_vega_kernel(StreamGeom g, SeedArgs seeds, ModelDev md, ScenDev sc, BookVega
         const float2 mask = make_float2(t.validA ? 1.0f : 0.0f, t.validB ? 1.0f : 0.0f);
         const bool full = __syncthreads_and(t.validA && t.validB);
 
-        // reference order: r, I of both twins of the base and of the two bumped scenarios; decomposed: the shared noise
-        float2 r1 = splat(md.r0), r2 = splat(md.r0), I1 = splat(0.0f), I2 = splat(0.0f);
-        PairState bp[2];
+        PairState tw[3];   // reference order: r, I of both twins of the three scenarios
 #pragma unroll
-        for (int s = 0; s < 2; ++s) {
-            bp[s].r1 = bp[s].r2 = splat(md.r0);
-            bp[s].I1 = bp[s].I2 = splat(0.0f);
+        for (int s = 0; s < 3; ++s) {
+            tw[s].r1 = tw[s].r2 = splat(md.r0);
+            tw[s].I1 = tw[s].I2 = splat(0.0f);
         }
-        FastState st;
-        st.h = splat(0.0f);
-        st.W = splat(0.0f);
-        int si = 0;   // steps taken (reference order: drift index)
-        auto step1 = [&](float2 G) {
-            if (DECOMP) {
-                st.W = add2(st.W, G);
-                st.h = fma2(st.h, e2, G);
-            } else {
-                const float2 d = splat(drift[si]);
-                hw_step2(r1, I1, fma2(G, sgP, d), e2, hdt2);
-                hw_step2(r2, I2, fma2(G, sgM, d), e2, hdt2);
+        auto ref_step = [&](float2 G, int si) {
 #pragma unroll
-                for (int s = 0; s < 2; ++s) {
-                    const float2 ds = splat(drift[(s + 1) * n_last + si]);
-                    hw_step2(bp[s].r1, bp[s].I1, fma2(G, sgPb[s], ds), e2, hdt2);
-                    hw_step2(bp[s].r2, bp[s].I2, fma2(G, sgMb[s], ds), e2, hdt2);
-                }
-            }
-            ++si;
-        };
-        // reference order: two steps per pair
-        auto pairfn = [&](int, float2 ns, float2 nc) { step1(ns); step1(nc); };
-        // decomposed: fast_kernel's pair step, the group's decay residual at HW1F_RHO_POS
-        auto fpair5 = [&](int j, float2 s, float2 sn, float2 c) {
-            const float2 a = fma2(sn, e2, c);
-            const float2 b = add2(sn, c);
-            if (j == HW1F_RHO_POS) st.h = fma2(st.h, splat(md.rho5), st.h);
-            st.h = fma2(s, a, mul2(st.h, ee2));
-            st.W = fma2(s, b, st.W);
-        };
-        auto fpair1 = [&](int, float2 s, float2 sn, float2 c) {
-            const float2 a = fma2(sn, e2, c);
-            const float2 b = add2(sn, c);
-            st.h = fma2(s, a, mul2(st.h, ee2));
-            st.W = fma2(s, b, st.W);
-        };
-        auto advance = [&](int n_pairs) {
-            if (DECOMP) {
-                int pair = 0, k = 0;
-                for (; k + 5 <= n_pairs; k += 5) { run_pairs_parts<5, 0>(t, pair, fpair5); pair += 5; }
-                for (; k < n_pairs; ++k) {
-                    st.h = fma2(st.h, splat(md.rho1), st.h);
-                    run_pairs_parts<1, 0>(t, pair, fpair1);
-                    pair += 1;
-                }
-                si += 2 * n_pairs;
-            } else {
-                int pair = 0;
-                advance_pairs(t, pair, n_pairs, pairfn);
+            for (int s = 0; s < 3; ++s) {
+                const float2 d = splat(drift[s * n_last + si]);
+                hw_step2(tw[s].r1, tw[s].I1, fma2(G, splat(sg[s]), d), e2, hdt2);
+                hw_step2(tw[s].r2, tw[s].I2, fma2(G, splat(-sg[s]), d), e2, hdt2);
             }
         };
-
-        bool pending = false;          // the cos half of the last pair is still to be stepped
-        float2 nc_keep = splat(0.0f);
-        if (lead) {                    // the launch starts on the cos half of a pair the previous launch opened
-            float2 ns;
-            one_pair(t, ns, nc_keep);
-            pending = true;
-        }
-        float2 Xs = splat(0.0f), Ys = splat(0.0f);   // book: sum of X_i and of the centred Y_i
+        float2 Xs = splat(0.0f), Ys = splat(0.0f);                       // book: sum of X_i and of the centred Y_i
         float2 Xms = splat(0.0f), Xps = splat(0.0f), Ds = splat(0.0f);   // book: sums of X-_i, X+_i, D_i
-        for (int i = 0; i < n; ++i) {
-            const SwaptionSh o = ss[i];
-            int left = o.step - si;
-            if (left > 0) {
-                if (pending) { step1(nc_keep); pending = false; --left; }
-                advance(left >> 1);
-                if (left & 1) {
-                    float2 ns;
-                    one_pair(t, ns, nc_keep);
-                    step1(ns);
-                    pending = true;
-                }
-            }
-            PairState ps, pb[2];
+        exercise_walk<DECOMP>(t, md, ss, fs, n, lead, ref_step,
+                              [&](int i, const SwaptionSh& o, const SwFlowSh& f0, const FastState& st) {
+            PairState ps = tw[0], pm = tw[1], pp = tw[2];
             if (DECOMP) {
                 const float2 q = st.q(md.qA, md.qB);
-                const float2 dr = mul2(st.h, splat(sc.sig_st)), dI = mul2(q, splat(cI));
-                ps.r1 = add2(splat(o.m), dr);
-                ps.r2 = add2(splat(o.m), make_float2(-dr.x, -dr.y));
-                ps.I1 = add2(splat(o.Im), dI);
-                ps.I2 = add2(splat(o.Im), make_float2(-dI.x, -dI.y));
                 const BookVegaOptDev b = bs[i];
-#pragma unroll
-                for (int s = 0; s < 2; ++s) {
-                    const float2 drs = mul2(st.h, splat(bv.sig_st[s])), dIs = mul2(q, splat(cIb[s]));
-                    pb[s].r1 = add2(splat(b.m[s]), drs);
-                    pb[s].r2 = add2(splat(b.m[s]), make_float2(-drs.x, -drs.y));
-                    pb[s].I1 = add2(splat(b.Im[s]), dIs);
-                    pb[s].I2 = add2(splat(b.Im[s]), make_float2(-dIs.x, -dIs.y));
-                }
-            } else {
-                ps.r1 = r1; ps.r2 = r2; ps.I1 = I1; ps.I2 = I2;
-                pb[0] = bp[0];
-                pb[1] = bp[1];
+                ps = rebuild_twins(st.h, q, o.m, o.Im, sg[0], cI[0]);
+                pm = rebuild_twins(st.h, q, b.m[0], b.Im[0], sg[1], cI[1]);
+                pp = rebuild_twins(st.h, q, b.m[1], b.Im[1], sg[2], cI[2]);
             }
             float2 x1, x2, y1, y2;
-            swaption_payoffs(ps, fs + o.f0, o.nf, o.K, o.sgn, x1, x2, y1, y2);
+            swaption_payoffs(ps, f0, fs + o.f0, o.nf, o.K, o.sgn, x1, x2, y1, y2);
             float2 X = mul2(splat(o.N), add2(x1, x2));
             float2 Y = add2(mul2(splat(o.N), add2(y1, y2)), splat(-o.cen));
             float2 xm1, xm2, xp1, xp2;
-            bumped_payoffs(pb[0], pb[1], fs + o.f0, fa + o.f0, o.nf, o.K, o.sgn, xm1, xm2, xp1, xp2);
+            bumped_payoffs(pm, pp, fs + o.f0, fa + o.f0, o.nf, o.K, o.sgn, xm1, xm2, xp1, xp2);
             float2 Xm = mul2(splat(o.N), add2(xm1, xm2));
             float2 Xp = mul2(splat(o.N), add2(xp1, xp2));
             if (!full) {   // block-uniform: ragged edge chunks only
@@ -285,63 +189,13 @@ book_vega_kernel(StreamGeom g, SeedArgs seeds, ModelDev md, ScenDev sc, BookVega
             Xms = add2(Xms, Xm);
             Xps = add2(Xps, Xp);
             Ds = add2(Ds, D);
-            {
-                const float sX = warp_sum_pair(add_(X.x, X.y), add_(Y.x, Y.y), lane);
-                const float sQ = warp_sum_pair(fma_(X.x, X.x, mul_(X.y, X.y)), fma_(Y.x, Y.x, mul_(Y.y, Y.y)), lane);
-                const float sXY = warp_sum(fma_(X.x, Y.x, mul_(X.y, Y.y)));
-                float* row = wflt + warp * nq + 5 * i + ((lane & 16) ? 1 : 0);
-                if (writer) { row[0] = sX; row[2] = sQ; }
-                if (lane == 0) row[4] = sXY;
-            }
-            {
-                const float sm = warp_sum_pair(add_(Xm.x, Xm.y), fma_(Xm.x, Xm.x, mul_(Xm.y, Xm.y)), lane);
-                const float sp = warp_sum_pair(add_(Xp.x, Xp.y), fma_(Xp.x, Xp.x, mul_(Xp.y, Xp.y)), lane);
-                const float sd = warp_sum_pair(add_(D.x, D.y), fma_(D.x, D.x, mul_(D.y, D.y)), lane);
-                float* row = wflt + warp * nq + nb + 6 * i + ((lane & 16) ? 1 : 0);
-                if (writer) { row[0] = sm; row[2] = sp; row[4] = sd; }
-            }
-        }
-        {
-            const float sX = warp_sum_pair(add_(Xs.x, Xs.y), add_(Ys.x, Ys.y), lane);
-            const float sQ = warp_sum_pair(fma_(Xs.x, Xs.x, mul_(Xs.y, Xs.y)), fma_(Ys.x, Ys.x, mul_(Ys.y, Ys.y)), lane);
-            const float sXY = warp_sum(fma_(Xs.x, Ys.x, mul_(Xs.y, Ys.y)));
-            float* row = wflt + warp * nq + 5 * n + ((lane & 16) ? 1 : 0);
-            if (writer) { row[0] = sX; row[2] = sQ; }
-            if (lane == 0) row[4] = sXY;
-        }
-        {
-            const float sm = warp_sum_pair(add_(Xms.x, Xms.y), fma_(Xms.x, Xms.x, mul_(Xms.y, Xms.y)), lane);
-            const float sp = warp_sum_pair(add_(Xps.x, Xps.y), fma_(Xps.x, Xps.x, mul_(Xps.y, Xps.y)), lane);
-            const float sd = warp_sum_pair(add_(Ds.x, Ds.y), fma_(Ds.x, Ds.x, mul_(Ds.y, Ds.y)), lane);
-            float* row = wflt + warp * nq + nb + 6 * n + ((lane & 16) ? 1 : 0);
-            if (writer) { row[0] = sm; row[2] = sp; row[4] = sd; }
-        }
+            write_moments5(wflt + warp * nq + 5 * i, X, Y, lane);
+            write_vega6(wflt + warp * nq + nb + 6 * i, Xm, Xp, D, lane);
+        });
+        write_moments5(wflt + warp * nq + 5 * n, Xs, Ys, lane);
+        write_vega6(wflt + warp * nq + nb + 6 * n, Xms, Xps, Ds, lane);
         __syncthreads();
-        // base, per option (and the book): sum the warp rows in double, undo the centring with this chunk's pair count
-        const unsigned long long base = (g.chunk0 + chunk) << kChunkLog2;
-        const unsigned long long lo = base > g.first_path ? base : g.first_path;
-        const unsigned long long hi = (base + kChunk < g.first_path + g.n_paths) ? base + kChunk : g.first_path + g.n_paths;
-        const double nvp = (double)(hi - lo);
-        for (int i = tid; i <= n; i += kThreads) {
-            double s[5];
-#pragma unroll
-            for (int k = 0; k < 5; ++k) {
-                double acc = (double)wflt[5 * i + k];
-#pragma unroll
-                for (int w = 1; w < kWarps; ++w) acc += (double)wflt[w * nq + 5 * i + k];
-                s[k] = acc;
-            }
-            double c = 0.0;
-            if (i < n) c = (double)ss[i].cen;
-            else
-                for (int j = 0; j < n; ++j) c += (double)ss[j].cen;
-            double* b = bacc + 5 * i;
-            b[0] += s[0];
-            b[1] += s[1] + nvp * c;
-            b[2] += s[2];
-            b[3] += s[3] + 2.0 * c * s[1] + nvp * c * c;
-            b[4] += s[4] + c * s[0];
-        }
+        fold_moments5(g, chunk, wflt, nq, ss, n, bacc);
         // bumped scenarios: raw sums, no centring
         for (int k = tid; k < nv; k += kThreads) {
             double acc = (double)wflt[nb + k];

@@ -1,8 +1,8 @@
-"""The cap / floor strip kernel (cap_kernel) at the edges of its schedule, geometry and model space, in both arithmetic
-modes: every segment length of the walk between reset steps (and so every split of the decomposed mode into 5-pair
-groups and single pairs), shared reset steps, every normal-offset parity, ragged path ranges, odd strides and step
-counts, weak mean reversion, the 100-caplet maximum on the longest grid, degenerate caplets, the host algebra and the
-state an engine carries across calls."""
+"""Cap / floor strips, priced as books of one-flow options by swaption_kernel, at the edges of their schedule, geometry
+and model space, in both arithmetic modes: every segment length of the walk between reset steps (and so every split of
+the decomposed mode into 5-pair groups and single pairs), shared reset steps, every normal-offset parity, ragged path
+ranges, odd strides and step counts, weak mean reversion, the 100-caplet maximum on the longest grid, degenerate
+caplets, the host algebra and the state an engine carries across calls."""
 import numpy as np
 import pytest
 

@@ -10,7 +10,8 @@ import re
 import subprocess
 import sys
 
-KERNELS = ("fast_kernel", "bond_curve_kernel", "zbc_kernel", "fused_kernel", "pathwise_kernel", "zbc_sum_kernel")
+KERNELS = ("fast_kernel", "bond_curve_kernel", "zbc_kernel", "fused_kernel", "pathwise_kernel", "zbc_sum_kernel",
+           "swaption_kernel", "book_vega_kernel")
 
 
 def functions(lib):
